@@ -2,7 +2,7 @@
 """bench.py -- the hot path's throughput on B200, one JSON line on stdout (rank 0).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--batch B]
-                    [--math parity|tf32|bf16] [--no-extras] [--no-cpu-baseline] [--no-graph]
+                    [--math parity|tf32|bf16] [--no-extras] [--no-cpu-baseline] [--no-graph] [--dump-outputs DIR]
 
 Headline (default workload `train`): BASELINE.json configs[1] -- ROBO-UNet 160x120 TRAINING, batch 64 per GPU, synthetic
 images/labels, 5 classes; a "step" is one full train step (forward, weighted CE, + L1 term, backward, Adam) over one
@@ -14,8 +14,13 @@ with its own e2e, whole-step roofline and CPU baseline, and at --gpus N > 1 the 
 
 --impl reference times the reference's own CPU implementation of the same step on the box's host cores: the
 UNMODIFIED reference classes from baseline/_ref/model.py when that staged copy exists (__graft_entry__.build() stages
-it where /root/reference exists; git-ignored), else the oracle port (oracle/ref_train.py drives the same ATen CPU
-kernels the reference's model.py dispatches to).
+it from oracle.reference_dir() where that checkout of the original project exists; git-ignored), else the oracle port
+(oracle/ref_train.py drives the same ATen CPU kernels the reference's model.py dispatches to).
+
+--dump-outputs DIR writes, on rank 0, what the timed loop's last step returned as DIR/<name>.npy (see dump_outputs): a
+training step's loss sums, L1 sum and correct-pixel count, an inference step's logits, loss, argmax, confusion,
+correct count and IoU sums.  Inputs and initial weights are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -291,6 +296,33 @@ def cpu_reference(wl, batch, steps, warmup, ckpt=None, budget_s=None):
     return batch / dt, dt * 1e3, threads, kind, n
 
 
+DUMP_MAX_ELEMS = 1 << 20        # per array: larger outputs are stored as a fixed, seeded sample of this many elements
+DUMP_MAX_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir, arrays: dict) -> None:
+    """arrays (name -> tensor) as out_dir/<name>.npy: floating point as float32 (float64 stays float64), integers as
+    float64 (exact below 2**53).  An array of more than DUMP_MAX_ELEMS elements is flattened and sampled at indices
+    drawn from a generator seeded with 0 (sorted), the same for every run of the same shape; smaller arrays keep
+    their shape."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMS].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        t = t.cpu()
+        host[name] = t.double() if t.dtype == torch.float64 or not t.is_floating_point() else t.float()
+    total = sum(t.numel() * t.element_size() for t in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    for name, t in host.items():
+        np.save(out_dir / f"{name}.npy", t.numpy())
+
+
 _REAL_STDOUT = None
 
 
@@ -335,8 +367,9 @@ class Job:
 
 
 def run_workload(job: Job, key: str, batch: int, steps: int, warmup: int, headline: bool, latency: bool = False,
-                 ckpt: str = None, cpu_budget_s: float = 3.0, math: str = None):
-    """One workload on this job's ranks -> record (dict).  Also returns the model for the headline's kernel rooflines."""
+                 ckpt: str = None, cpu_budget_s: float = 3.0, math: str = None, dump_dir: str = None):
+    """One workload on this job's ranks -> record (dict).  Also returns the model for the headline's kernel rooflines.
+    dump_dir: write the last timed step's outputs there (dump_outputs)."""
     from robocupvision_b200 import _lib, ops
     from robocupvision_b200.train import EvalStep, TrainStep
     args, dev, world, rank = job.args, job.dev, job.world, job.rank
@@ -376,6 +409,15 @@ def run_workload(job: Job, key: str, batch: int, steps: int, warmup: int, headli
     job.barrier()
     ms_total = job.max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / steps
+    if dump_dir is not None and rank == 0:
+        # what TrainStep.step / EvalStep return, read before anything else runs the model again.  The weights a
+        # training step leaves behind are not dumped: weight-gradient atomics and ReLU sign flips make them drift
+        # between identical runs (DESIGN.md section 2), far more than the loss does
+        if wl["train"]:
+            res = {"loss_sums": ts.loss_sums, "l1_sum": ts.l1_sum, "correct": ts.correct}
+        else:
+            res = dict(out["r"])
+        dump_outputs(dump_dir, res)
     extra_steps = 0
     if headline:
         # a timed region shorter than a few sampling periods: keep the same load running (untimed) until three
@@ -504,7 +546,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--extra-steps", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference arm only times")
     if args.math != "parity":
         os.environ["RCV_B200_MATH"] = args.math
     wl = WORKLOADS[args.workload]
@@ -518,11 +566,10 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        # bounded: the CPU step is 0.2-2 s; same --steps / --warmup as the repo arm up to a cap that keeps the run
-        # within a few minutes
-        steps, warm = max(1, min(args.steps, 60)), max(1, min(args.warmup, 10))
+        # exactly --steps timed steps after --warmup untimed ones (a CPU step takes 0.2-2 s)
+        steps, warm = args.steps, args.warmup
         cb = min(batch, 64)
-        fps, ms, threads, kind, n = cpu_reference(wl, cb, steps, warm, wl.get("ckpt"), budget_s=150.0)
+        fps, ms, threads, kind, n = cpu_reference(wl, cb, steps, warm, wl.get("ckpt"))
         sample = (f"{n} steps of batch {cb} after {warm} warm-up ("
                   + ("the unmodified reference classes, baseline/_ref/model.py" if kind == "reference" else "oracle port")
                   + f", torch {torch.__version__} CPU)")
@@ -550,7 +597,8 @@ def main():
         job.sampler = ClockSampler(job.local_rank)
         job.sampler.start()
 
-    rec, model = run_workload(job, args.workload, batch, args.steps, args.warmup, headline=True)
+    rec, model = run_workload(job, args.workload, batch, args.steps, args.warmup, headline=True,
+                              dump_dir=args.dump_outputs)
     row0, row1, extra_steps = rec.pop("_clock_rows")
     clocks = job.sampler.summary(row0, row1) if job.sampler else {"sm_mhz": None, "sm_max_mhz": None, "reasons": []}
     clocks["window"] = "timed region" if extra_steps == 0 else f"timed region + {extra_steps} untimed steps of the same load"

@@ -14,6 +14,13 @@ ROBO_VARIANTS = {
     "robo_noscale": (dict(noScale=True), dict(no_scale=True)),
 }
 
+# (class name, args, kwargs) of the module trees pinned against the original project's classes
+# (tests/golden/reference_module_tree.json, oracle/make_golden_classes.py)
+TREE_CASES = ([("ROBO_UNet", (), kw) for kw, _ in ROBO_VARIANTS.values()]
+              + [("ROBO_UNet", (), dict(v2=True, levels=1, bellySize=9, classSize=3, bellyPlanes=64))]
+              + [("PB_FCN", (32, 5, 1, ns, 0), {}) for ns in (False, True)]
+              + [("FCN", (), {}), ("DownSampler", (32, False), {})])
+
 
 def robo_state(tag):
     """Seed 12345678 init (train.py:332-337) + three oracle training forwards so the running
