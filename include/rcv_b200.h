@@ -461,6 +461,55 @@ int rcv_sgd_step(int64_t n, float* p, const float* g, float* buf,
  * arena (optimizer.zero_grad(), train.py:45), BatchNorm statistics, loss sums. */
 int rcv_zero(void* ptr, size_t bytes, void* stream);
 
+/* ---- deterministic (fixed-order) reductions ------------------------------ */
+/* The entry points above add each CTA's partial sums into their destination with floating-point atomics, so the
+ * order of the additions, and the last bits of the result, change from run to run.  Each _det variant below computes
+ * exactly what its plain form computes, with one difference: every CTA parks its partial vector in a slot of
+ * `scratch` fixed by the launch geometry, and the CTA that arrives last adds the slots into the destination in an
+ * order fixed by the launch geometry (never by the arrival order).  Same inputs on the same device: bitwise the same result, run after run (torch.use_deterministic_algorithms,
+ * the reference's seeded CPU runs).  It differs from the plain form in summation order only.
+ * scratch: caller-owned device memory of at least rcv_det_scratch_bytes(op, ...) bytes, 128-byte aligned,
+ * ZERO-FILLED ONCE by the caller before its first use (the kernels leave it ready for the next call), used by one
+ * stream at a time; too small is RCV_ERR_WORKSPACE.  The scratch needed depends on the grid, which follows the
+ * problem size and the device. */
+typedef enum rcv_det_op {
+  RCV_DET_CE_FWD = 0,         /* rcv_ce_fwd_det: N images of HW pixels (C ignored)                  */
+  RCV_DET_CE_WEIGHT_SUM = 1,  /* rcv_ce_weight_sum_det: count = N*HW labels (C ignored)             */
+  RCV_DET_DICE_FWD = 2,       /* rcv_dice_fwd_det: N images of HW pixels, C classes                 */
+  RCV_DET_L1_SUM = 3          /* rcv_adam_l1_step_det / rcv_sgd_step_det: n = N*HW parameters      */
+} rcv_det_op;
+/* Bytes of scratch the _det entry point of `op` needs for this problem; 0 for an unknown op or a problem the entry
+ * point refuses.  Host only: needs no GPU. */
+size_t rcv_det_scratch_bytes(int op, int32_t N, int32_t C, int64_t HW);
+
+/* rcv_ce_fwd with loss_sums in fixed order: CrossEntropyLoss2d (model.py:76-82).  argmax / conf / correct are integer counts and exact either way.  scratch may be NULL when
+ * loss_sums is NULL. */
+int rcv_ce_fwd_det(int32_t N, int32_t C, int64_t HW, const float* logits,
+                   const int64_t* target, const float* class_w, double* loss_sums,
+                   int64_t* argmax, int64_t* conf, int64_t* correct, void* scratch,
+                   uint64_t scratch_bytes, void* stream);
+/* rcv_ce_weight_sum in fixed order: the normaliser sum_p w[y_p] of CrossEntropyLoss2d's weighted mean
+ * (model.py:76-82); the atomic form is exact only when the class weights are integers. */
+int rcv_ce_weight_sum_det(int32_t C, int64_t count, const int64_t* target, const float* class_w,
+                          double* out, void* scratch, uint64_t scratch_bytes, void* stream);
+/* rcv_dice_fwd in fixed order: DiceLoss's intersection and cardinality sums (model.py:5-43). */
+int rcv_dice_fwd_det(int32_t N, int32_t C, int64_t HW, const float* logits,
+                     const int64_t* target, double* sums, void* scratch,
+                     uint64_t scratch_bytes, void* stream);
+/* rcv_adam_l1_step / rcv_sgd_step with l1_sum in fixed order: the L1 term the reference adds to the reported loss
+ * (train.py:23-27).  The parameter updates are element-wise and identical to the plain forms.  scratch may be
+ * NULL when l1_sum is NULL. */
+int rcv_adam_l1_step_det(int64_t n, float* p, const float* g, float* m, float* v,
+                         const uint8_t* mask, float lr, float beta1, float beta2,
+                         float eps, int32_t step, float l1_decay, float grad_scale,
+                         double* l1_sum, const int32_t* step_dev, const float* lr_dev,
+                         void* scratch, uint64_t scratch_bytes, void* stream);
+int rcv_sgd_step_det(int64_t n, float* p, const float* g, float* buf,
+                     const uint8_t* mask, float lr, float momentum,
+                     float weight_decay, float grad_scale, int first_step,
+                     float l1_decay, double* l1_sum, const float* lr_dev,
+                     void* scratch, uint64_t scratch_bytes, void* stream);
+
 /* ---- data-parallel gradient exchange over NVLink peer memory ------------- */
 /* The one exchange of batch-sharded training: the sum all-reduce of the flat gradient arena after
  * `loss.backward()` (train.py:66; what DistributedDataParallel adds to the reference's loop), as ONE kernel per

@@ -32,6 +32,8 @@ RCV_OK, RCV_ERR_BAD_ARG, RCV_ERR_UNSUPPORTED, RCV_ERR_CUDA, RCV_ERR_WORKSPACE = 
 EPI_NONE, EPI_RELU, EPI_RELU_AFFINE, EPI_AFFINE_RELU, EPI_AFFINE = 0, 1, 2, 3, 4
 # rcv_math
 MATH_FP32, MATH_TF32X3, MATH_AUTO, MATH_TF32, MATH_BF16 = 0, 1, 2, 3, 4
+# rcv_det_op
+DET_CE_FWD, DET_CE_WEIGHT_SUM, DET_DICE_FWD, DET_L1_SUM = 0, 1, 2, 3
 # rcv_engine
 ENGINE_SIMT, ENGINE_DIRECT, ENGINE_UMMA, ENGINE_NARROW = 0, 1, 2, 3
 
@@ -109,9 +111,17 @@ SIGNATURES = {
     "rcv_counter_add": [_p, _i32, _p],
     "rcv_sgd_step": [_i64, _p, _p, _p, _p, _f32, _f32, _f32, _f32, C.c_int, _f32, _p, _p, _p],
     "rcv_zero": [_p, C.c_size_t, _p],
+    "rcv_det_scratch_bytes": [C.c_int, _i32, _i32, _i64],
+    "rcv_ce_fwd_det": [_i32, _i32, _i64, _p, _p, _p, _p, _p, _p, _p, _p, C.c_uint64, _p],
+    "rcv_ce_weight_sum_det": [_i32, _i64, _p, _p, _p, _p, C.c_uint64, _p],
+    "rcv_dice_fwd_det": [_i32, _i32, _i64, _p, _p, _p, _p, C.c_uint64, _p],
+    "rcv_adam_l1_step_det": [_i64, _p, _p, _p, _p, _p, _f32, _f32, _f32, _f32, _i32, _f32, _f32, _p, _p, _p, _p,
+                             C.c_uint64, _p],
+    "rcv_sgd_step_det": [_i64, _p, _p, _p, _p, _f32, _f32, _f32, _f32, C.c_int, _f32, _p, _p, _p, C.c_uint64, _p],
 }
 _RESTYPES = {"rcv_last_error": C.c_char_p, "rcv_conv_packed_bytes": C.c_size_t, "rcv_conv_workspace_bytes": C.c_size_t,
-             "rcv_conv_pack_table_bytes": C.c_size_t, "rcv_peer_flag_bytes": C.c_uint64}
+             "rcv_conv_pack_table_bytes": C.c_size_t, "rcv_peer_flag_bytes": C.c_uint64,
+             "rcv_det_scratch_bytes": C.c_size_t}
 PACK_FWD, PACK_DGRAD = 0, 1
 ABI_VERSION = 5
 

@@ -21,6 +21,17 @@ long long* g_rcv_prof = nullptr;
 extern "C" void rcv_debug_set_prof(void* buf) { g_rcv_prof = reinterpret_cast<long long*>(buf); }
 
 extern "C" int rcv_version(void) { return RCV_ABI_VERSION; }
+
+extern "C" size_t rcv_det_scratch_bytes(int op, int32_t N, int32_t C, int64_t HW) {
+  if (N <= 0 || HW <= 0) return 0;
+  switch (op) {
+    case RCV_DET_CE_FWD: return N <= 65535 ? rcv_ce_fwd_det_bytes(N, HW) : 0;
+    case RCV_DET_CE_WEIGHT_SUM: return rcv_ce_weight_sum_det_bytes((int64_t)N * HW);
+    case RCV_DET_DICE_FWD: return N <= 65535 && C >= 2 && C <= 8 ? rcv_dice_fwd_det_bytes(N, C, HW) : 0;
+    case RCV_DET_L1_SUM: return rcv_l1_sum_det_bytes((int64_t)N * HW);
+    default: return 0;
+  }
+}
 extern "C" const char* rcv_last_error(void) { return g_err; }
 
 namespace {

@@ -61,10 +61,12 @@ __device__ __forceinline__ void softmax_px(const float* __restrict__ lp, int64_t
   for (int c = 0; c < C; ++c) s[c] *= inv;
 }
 
-// sums[c] += sum_p softmax_c(p) * [y_p == c];  sums[C + c] += sum_p (softmax_c(p) + [y_p == c])
-template <int C>
+// sums[c] += sum_p softmax_c(p) * [y_p == c];  sums[C + c] += sum_p (softmax_c(p) + [y_p == c]).
+// DET: added into sums through the ordered flush over det (slot = linear block index) instead of atomics.
+template <int C, bool DET = false>
 __global__ void __launch_bounds__(NT) dice_fwd_kernel(int64_t HW, const float* __restrict__ logits,
-                                                       const long long* __restrict__ target, double* sums) {
+                                                       const long long* __restrict__ target, double* sums,
+                                                       void* det) {
   rcv_pdl_enter();
   __shared__ double red[2 * CMAX][NT / 32];
   const int n = blockIdx.y;
@@ -102,11 +104,17 @@ __global__ void __launch_bounds__(NT) dice_fwd_kernel(int64_t HW, const float* _
     if (l == 0) { red[c][wi] = a; red[CMAX + c][wi] = b; }
   }
   __syncthreads();
+  double t = 0.0;
   if (threadIdx.x < 2 * C) {
     const int which = threadIdx.x / C, c = threadIdx.x - which * C;
-    double t = 0.0;
     for (int w = 0; w < NT / 32; ++w) t += red[which * CMAX + c][w];
-    atomicAdd(sums + which * C + c, t);
+    if constexpr (!DET) atomicAdd(sums + which * C + c, t);
+  }
+  if constexpr (DET) {
+    __syncthreads();  // every row of red is read before red holds this CTA's partial, sums[] order
+    if (threadIdx.x < 2 * C) (&red[0][0])[threadIdx.x] = t;
+    __syncthreads();
+    rcv_ordered_flush(det, blockIdx.y * gridDim.x + blockIdx.x, gridDim.x * gridDim.y, 2 * C, &red[0][0], sums);
   }
 }
 
@@ -177,18 +185,47 @@ extern "C" int rcv_augment(int32_t N, int32_t H, int32_t W, const float* x, floa
   return RCV_OK;
 }
 
-extern "C" int rcv_dice_fwd(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
-                            double* sums, void* stream) {
+namespace {
+dim3 dice_grid(int32_t N, int64_t HW) {
+  const int bx = rcv_cdiv(148 * 8, N);
+  return dim3(blocks_for(HW, bx < 1 ? 1 : bx), N);
+}
+
+int dice_fwd_launch(bool det, int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
+                    double* sums, void* scratch, void* stream) {
   RCV_REQUIRE(N > 0 && HW > 0 && logits && target && sums, RCV_ERR_BAD_ARG, "dice_fwd: bad arg");
   RCV_REQUIRE(C >= 2 && C <= CMAX, RCV_ERR_UNSUPPORTED, "dice_fwd: C=%d (supported 2..8)", C);
   RCV_REQUIRE(N <= 65535, RCV_ERR_UNSUPPORTED, "dice_fwd: N=%d > 65535", N);
-  int bx = rcv_cdiv(148 * 8, N);
-  dim3 grid(blocks_for(HW, bx < 1 ? 1 : bx), N);
+  const dim3 grid = dice_grid(N, HW);
   cudaStream_t st = (cudaStream_t)stream;
-  RCV_DICE_DISPATCH(C, (rcv_launch(dice_fwd_kernel<CC>, dim3(grid), dim3(NT), 0, st, HW, logits,
-                                   reinterpret_cast<const long long*>(target), sums)));
+  const long long* tg = reinterpret_cast<const long long*>(target);
+  if (det) {
+    RCV_DICE_DISPATCH(C, (rcv_launch(dice_fwd_kernel<CC, true>, grid, dim3(NT), 0, st, HW, logits, tg, sums, scratch)));
+  } else {
+    RCV_DICE_DISPATCH(C, (rcv_launch(dice_fwd_kernel<CC>, grid, dim3(NT), 0, st, HW, logits, tg, sums, scratch)));
+  }
   RCV_CHECK_LAUNCH("dice_fwd");
   return RCV_OK;
+}
+}  // namespace
+
+extern "C" int rcv_dice_fwd(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
+                            double* sums, void* stream) {
+  return dice_fwd_launch(false, N, C, HW, logits, target, sums, nullptr, stream);
+}
+
+size_t rcv_dice_fwd_det_bytes(int32_t N, int32_t C, int64_t HW) {
+  const dim3 g = dice_grid(N, HW);
+  return rcv_det_bytes((long long)g.x * g.y, 2 * C, sizeof(double));
+}
+
+extern "C" int rcv_dice_fwd_det(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
+                                double* sums, void* scratch, uint64_t scratch_bytes, void* stream) {
+  RCV_REQUIRE(N > 0 && N <= 65535 && HW > 0 && C >= 2 && C <= CMAX, RCV_ERR_BAD_ARG, "dice_fwd_det: bad arg");
+  RCV_REQUIRE(scratch && scratch_bytes >= rcv_dice_fwd_det_bytes(N, C, HW), RCV_ERR_WORKSPACE,
+              "dice_fwd_det: scratch of %llu bytes, %zu needed", (unsigned long long)scratch_bytes,
+              rcv_dice_fwd_det_bytes(N, C, HW));
+  return dice_fwd_launch(true, N, C, HW, logits, target, sums, scratch, stream);
 }
 
 extern "C" int rcv_dice_bwd(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,

@@ -48,6 +48,66 @@ __device__ __forceinline__ void rcv_pdl_enter() {
 
 bool rcv_pdl_enabled();  // RCV_PDL (rcv_api.cu)
 
+// ---------------------------------------------------------------------------
+// Ordered flush: the fixed-order replacement of "every CTA atomically adds its partial vector into dst" used by the
+// deterministic (_det) entry points.  Scratch layout (caller-owned, rcv_det_scratch_bytes): a uint32 arrival
+// counter padded to RCV_DET_COUNTER_BYTES, then T partials[nslots][len].  128-byte aligned, zero-filled once by the
+// caller, left with its counter zeroed again, one stream at a time -- the convention of rcv_conv_desc::workspace.
+// ---------------------------------------------------------------------------
+constexpr size_t RCV_DET_COUNTER_BYTES = 128;
+
+static inline size_t rcv_det_bytes(long long nslots, long long len, size_t elem) {
+  return RCV_DET_COUNTER_BYTES + (((size_t)nslots * (size_t)len * elem + 127) & ~(size_t)127);
+}
+
+// scratch each deterministic entry point needs (rcv_det_scratch_bytes)
+size_t rcv_ce_fwd_det_bytes(int32_t N, int64_t HW);
+size_t rcv_ce_weight_sum_det_bytes(int64_t count);
+size_t rcv_dice_fwd_det_bytes(int32_t N, int32_t C, int64_t HW);
+size_t rcv_l1_sum_det_bytes(int64_t n);
+
+#ifdef __CUDACC__
+// Called by every thread of the CTA (no early exits before it).  mine[0..len) (shared memory, or any memory every
+// thread of the CTA can read) is this CTA's partial vector; slot comes from the launch geometry, never from the
+// arrival order.  Each CTA parks its partial in its slot and takes a ticket; the one that arrives last adds up the
+// slots and adds the total into dst (dst[i] += total, as the atomic form does), then resets the counter.  The order
+// of the additions depends on nslots and blockDim.x only: thread t sums slots t, t + blockDim.x, ... in turn, the
+// threads of a warp combine by a fixed butterfly, and thread 0 adds the warp sums in warp order -- the last CTA's
+// whole block shares the work, so the tail stays short at a thousand slots.  No CTA waits for another, so CTAs that
+// are not resident at the same time cannot deadlock it.  The memory ordering is that of the split reduction of the
+// halo-staged tensor-core kernel (rcv_umma_halo.cu, split_exchange).  blockDim.x: a multiple of 32, at most 1024.
+template <typename T>
+__device__ __noinline__ void rcv_ordered_flush(void* scratch, int slot, int nslots, int len, const T* mine, T* dst) {
+  __shared__ uint32_t s_ticket;
+  __shared__ T s_warp[32];
+  uint32_t* counter = reinterpret_cast<uint32_t*>(scratch);
+  T* parts = reinterpret_cast<T*>(reinterpret_cast<unsigned char*>(scratch) + RCV_DET_COUNTER_BYTES);
+  for (int i = threadIdx.x; i < len; i += blockDim.x) __stcg(parts + (size_t)slot * len + i, mine[i]);
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_ticket = atomicAdd(counter, 1u);
+  __syncthreads();
+  if (s_ticket != (uint32_t)(nslots - 1)) return;
+  __threadfence();
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  for (int i = 0; i < len; ++i) {
+    T t = T(0);
+    for (int s = threadIdx.x; s < nslots; s += blockDim.x) t += __ldcg(parts + (size_t)s * len + i);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+    if (lane == 0) s_warp[warp] = t;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      T u = s_warp[0];
+      for (int w = 1; w < nwarps; ++w) u += s_warp[w];
+      dst[i] += u;
+    }
+    __syncthreads();  // s_warp is reused by the next element
+  }
+  if (threadIdx.x == 0) *counter = 0u;  // every slot has arrived: ready for the next launch
+}
+#endif
+
 // The one way kernels are launched: plain stream order, or programmatic dependent launch when enabled.  Errors
 // are picked up by RCV_CHECK_LAUNCH right after.
 template <typename... KArgs, typename... Args>

@@ -42,9 +42,11 @@ __device__ __forceinline__ void stv(float* p, const float (&o)[VEC]) {
   *reinterpret_cast<typename VecT<VEC>::F*>(p) = v;
 }
 
-// sum over all pixels of class_w[target] (1 without weights): the normaliser of the mean-reduced weighted loss
+// sum over all pixels of class_w[target] (1 without weights): the normaliser of the mean-reduced weighted loss.
+// DET: added into out through the ordered flush over det (slot = block index) instead of an atomic.
+template <bool DET>
 __global__ void __launch_bounds__(NT) ce_wsum_kernel(int64_t count, int C, const int64_t* __restrict__ target,
-                                                     const float* __restrict__ class_w, double* out) {
+                                                     const float* __restrict__ class_w, double* out, void* det) {
   rcv_pdl_enter();
   __shared__ double sh[NT / 32];
   __shared__ float s_w[CMAX];
@@ -63,7 +65,12 @@ __global__ void __launch_bounds__(NT) ce_wsum_kernel(int64_t count, int C, const
   if (threadIdx.x == 0) {
     double t = 0.0;
     for (int i = 0; i < NT / 32; ++i) t += sh[i];
-    atomicAdd(out, t);
+    if constexpr (DET) sh[0] = t;
+    else atomicAdd(out, t);
+  }
+  if constexpr (DET) {
+    __syncthreads();
+    rcv_ordered_flush(det, blockIdx.x, gridDim.x, 1, sh, out);
   }
 }
 
@@ -247,16 +254,39 @@ extern "C" int rcv_head_ce_supported(int32_t Cin, int32_t C) {
   return (Cin == 8 || Cin == 16) && C >= 2 && C <= CMAX ? 1 : 0;
 }
 
-extern "C" int rcv_ce_weight_sum(int32_t C, int64_t count, const int64_t* target, const float* class_w, double* out,
-                                 void* stream) {
-  RCV_REQUIRE(count > 0 && target && out, RCV_ERR_BAD_ARG, "ce_weight_sum: bad arg");
-  RCV_REQUIRE(C >= 1 && C <= CMAX, RCV_ERR_UNSUPPORTED, "ce_weight_sum: C=%d (supported 1..8)", C);
+namespace {
+int ce_wsum_blocks(int64_t count) {
   int64_t nb = (count + NT * 8 - 1) / (NT * 8);
   if (nb > 148 * 4) nb = 148 * 4;
   if (nb < 1) nb = 1;
-  rcv_launch(ce_wsum_kernel, dim3((unsigned)nb), dim3(NT), 0, (cudaStream_t)stream, count, (int)C, target, class_w, out);
+  return (int)nb;
+}
+
+int ce_wsum_launch(bool det, int32_t C, int64_t count, const int64_t* target, const float* class_w, double* out,
+                   void* scratch, void* stream) {
+  RCV_REQUIRE(count > 0 && target && out, RCV_ERR_BAD_ARG, "ce_weight_sum: bad arg");
+  RCV_REQUIRE(C >= 1 && C <= CMAX, RCV_ERR_UNSUPPORTED, "ce_weight_sum: C=%d (supported 1..8)", C);
+  rcv_launch(det ? ce_wsum_kernel<true> : ce_wsum_kernel<false>, dim3((unsigned)ce_wsum_blocks(count)), dim3(NT), 0,
+             (cudaStream_t)stream, count, (int)C, target, class_w, out, scratch);
   RCV_CHECK_LAUNCH("ce_weight_sum");
   return RCV_OK;
+}
+}  // namespace
+
+extern "C" int rcv_ce_weight_sum(int32_t C, int64_t count, const int64_t* target, const float* class_w, double* out,
+                                 void* stream) {
+  return ce_wsum_launch(false, C, count, target, class_w, out, nullptr, stream);
+}
+
+size_t rcv_ce_weight_sum_det_bytes(int64_t count) { return rcv_det_bytes(ce_wsum_blocks(count), 1, sizeof(double)); }
+
+extern "C" int rcv_ce_weight_sum_det(int32_t C, int64_t count, const int64_t* target, const float* class_w,
+                                     double* out, void* scratch, uint64_t scratch_bytes, void* stream) {
+  RCV_REQUIRE(count > 0, RCV_ERR_BAD_ARG, "ce_weight_sum_det: bad arg");
+  RCV_REQUIRE(scratch && scratch_bytes >= rcv_ce_weight_sum_det_bytes(count), RCV_ERR_WORKSPACE,
+              "ce_weight_sum_det: scratch of %llu bytes, %zu needed", (unsigned long long)scratch_bytes,
+              rcv_ce_weight_sum_det_bytes(count));
+  return ce_wsum_launch(true, C, count, target, class_w, out, scratch, stream);
 }
 
 extern "C" int rcv_head_ce_train(int32_t N, int32_t Cin, int32_t C, int64_t HW, const float* feat, const float* weight,

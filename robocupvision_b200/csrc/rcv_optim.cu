@@ -7,6 +7,8 @@ namespace {
 
 constexpr int NT = 256;
 
+// DET (both kernels): l1_sum through the ordered flush over det (slot = block index) instead of an atomic.
+template <bool DET>
 __global__ void __launch_bounds__(NT) adam_l1_kernel(int64_t n, float* __restrict__ p,
                                                       const float* __restrict__ g,
                                                       float* __restrict__ m, float* __restrict__ v,
@@ -15,7 +17,7 @@ __global__ void __launch_bounds__(NT) adam_l1_kernel(int64_t n, float* __restric
                                                       float bc2_sqrt, float l1_decay, float grad_scale,
                                                       double* l1_sum,
                                                       const int32_t* __restrict__ step_dev,
-                                                      const float* __restrict__ lr_dev) {
+                                                      const float* __restrict__ lr_dev, void* det) {
   rcv_pdl_enter();
   __shared__ double sh[NT / 32];
   const int64_t stride = (int64_t)gridDim.x * NT;
@@ -51,17 +53,23 @@ __global__ void __launch_bounds__(NT) adam_l1_kernel(int64_t n, float* __restric
     if (threadIdx.x == 0) {
       double t = 0.0;
       for (int i = 0; i < NT / 32; ++i) t += sh[i];
-      atomicAdd(l1_sum, t);
+      if constexpr (DET) sh[0] = t;
+      else atomicAdd(l1_sum, t);
+    }
+    if constexpr (DET) {
+      __syncthreads();
+      rcv_ordered_flush(det, blockIdx.x, gridDim.x, 1, sh, l1_sum);
     }
   }
 }
 
+template <bool DET>
 __global__ void __launch_bounds__(NT) sgd_kernel(int64_t n, float* __restrict__ p,
                                                   const float* __restrict__ g, float* __restrict__ buf,
                                                   const uint8_t* __restrict__ mask, float lr,
                                                   float momentum, float wd, float grad_scale,
                                                   int first_step, float l1_decay, double* l1_sum,
-                                                  const float* __restrict__ lr_dev) {
+                                                  const float* __restrict__ lr_dev, void* det) {
   rcv_pdl_enter();
   __shared__ double sh[NT / 32];
   const int64_t stride = (int64_t)gridDim.x * NT;
@@ -90,7 +98,12 @@ __global__ void __launch_bounds__(NT) sgd_kernel(int64_t n, float* __restrict__ 
     if (threadIdx.x == 0) {
       double t = 0.0;
       for (int i = 0; i < NT / 32; ++i) t += sh[i];
-      atomicAdd(l1_sum, t);
+      if constexpr (DET) sh[0] = t;
+      else atomicAdd(l1_sum, t);
+    }
+    if constexpr (DET) {
+      __syncthreads();
+      rcv_ordered_flush(det, blockIdx.x, gridDim.x, 1, sh, l1_sum);
     }
   }
 }
@@ -104,19 +117,46 @@ int blocks_for(int64_t n) {
 
 }  // namespace
 
-extern "C" int rcv_adam_l1_step(int64_t n, float* p, const float* g, float* m, float* v,
-                                const uint8_t* mask, float lr, float beta1, float beta2, float eps,
-                                int32_t step, float l1_decay, float grad_scale, double* l1_sum,
-                                const int32_t* step_dev, const float* lr_dev, void* stream) {
+namespace {
+int adam_launch(bool det, int64_t n, float* p, const float* g, float* m, float* v, const uint8_t* mask, float lr,
+                float beta1, float beta2, float eps, int32_t step, float l1_decay, float grad_scale, double* l1_sum,
+                const int32_t* step_dev, const float* lr_dev, void* scratch, void* stream) {
   RCV_REQUIRE(n > 0 && p && g && m && v && (step >= 1 || step_dev), RCV_ERR_BAD_ARG,
               "adam_l1_step: bad arg");
   if (step < 1) step = 1;
   const double bc1 = 1.0 - pow((double)beta1, (double)step);
   const double bc2 = 1.0 - pow((double)beta2, (double)step);
-  rcv_launch(adam_l1_kernel, dim3(blocks_for(n)), dim3(NT), 0, (cudaStream_t)stream, n, p, g, m, v, mask, lr, beta1,
-             beta2, eps, (float)bc1, (float)sqrt(bc2), l1_decay, grad_scale, l1_sum, step_dev, lr_dev);
+  rcv_launch(det ? adam_l1_kernel<true> : adam_l1_kernel<false>, dim3(blocks_for(n)), dim3(NT), 0,
+             (cudaStream_t)stream, n, p, g, m, v, mask, lr, beta1, beta2, eps, (float)bc1, (float)sqrt(bc2), l1_decay,
+             grad_scale, l1_sum, step_dev, lr_dev, scratch);
   RCV_CHECK_LAUNCH("adam_l1_step");
   return RCV_OK;
+}
+}  // namespace
+
+extern "C" int rcv_adam_l1_step(int64_t n, float* p, const float* g, float* m, float* v,
+                                const uint8_t* mask, float lr, float beta1, float beta2, float eps,
+                                int32_t step, float l1_decay, float grad_scale, double* l1_sum,
+                                const int32_t* step_dev, const float* lr_dev, void* stream) {
+  return adam_launch(false, n, p, g, m, v, mask, lr, beta1, beta2, eps, step, l1_decay, grad_scale, l1_sum, step_dev,
+                     lr_dev, nullptr, stream);
+}
+
+size_t rcv_l1_sum_det_bytes(int64_t n) { return rcv_det_bytes(blocks_for(n), 1, sizeof(double)); }
+
+#define RCV_L1_SCRATCH_CHECK(name)                                                                                 \
+  RCV_REQUIRE(n > 0, RCV_ERR_BAD_ARG, name ": bad arg");                                                           \
+  RCV_REQUIRE(!l1_sum || (scratch && scratch_bytes >= rcv_l1_sum_det_bytes(n)), RCV_ERR_WORKSPACE,                 \
+              name ": scratch of %llu bytes, %zu needed", (unsigned long long)scratch_bytes, rcv_l1_sum_det_bytes(n))
+
+extern "C" int rcv_adam_l1_step_det(int64_t n, float* p, const float* g, float* m, float* v,
+                                    const uint8_t* mask, float lr, float beta1, float beta2, float eps,
+                                    int32_t step, float l1_decay, float grad_scale, double* l1_sum,
+                                    const int32_t* step_dev, const float* lr_dev, void* scratch,
+                                    uint64_t scratch_bytes, void* stream) {
+  RCV_L1_SCRATCH_CHECK("adam_l1_step_det");
+  return adam_launch(true, n, p, g, m, v, mask, lr, beta1, beta2, eps, step, l1_decay, grad_scale, l1_sum, step_dev,
+                     lr_dev, scratch, stream);
 }
 
 __global__ void counter_add_kernel(int32_t* c, int32_t inc) { rcv_pdl_enter(); *c += inc; }
@@ -128,15 +168,33 @@ extern "C" int rcv_counter_add(int32_t* counter, int32_t inc, void* stream) {
   return RCV_OK;
 }
 
+namespace {
+int sgd_launch(bool det, int64_t n, float* p, const float* g, float* buf, const uint8_t* mask, float lr,
+               float momentum, float weight_decay, float grad_scale, int first_step, float l1_decay, double* l1_sum,
+               const float* lr_dev, void* scratch, void* stream) {
+  RCV_REQUIRE(n > 0 && p && g && (momentum == 0.f || buf), RCV_ERR_BAD_ARG, "sgd_step: bad arg");
+  rcv_launch(det ? sgd_kernel<true> : sgd_kernel<false>, dim3(blocks_for(n)), dim3(NT), 0, (cudaStream_t)stream, n,
+             p, g, buf, mask, lr, momentum, weight_decay, grad_scale, first_step, l1_decay, l1_sum, lr_dev, scratch);
+  RCV_CHECK_LAUNCH("sgd_step");
+  return RCV_OK;
+}
+}  // namespace
+
 extern "C" int rcv_sgd_step(int64_t n, float* p, const float* g, float* buf, const uint8_t* mask,
                             float lr, float momentum, float weight_decay, float grad_scale,
                             int first_step, float l1_decay, double* l1_sum, const float* lr_dev,
                             void* stream) {
-  RCV_REQUIRE(n > 0 && p && g && (momentum == 0.f || buf), RCV_ERR_BAD_ARG, "sgd_step: bad arg");
-  rcv_launch(sgd_kernel, dim3(blocks_for(n)), dim3(NT), 0, (cudaStream_t)stream, n, p, g, buf, mask, lr, momentum,
-             weight_decay, grad_scale, first_step, l1_decay, l1_sum, lr_dev);
-  RCV_CHECK_LAUNCH("sgd_step");
-  return RCV_OK;
+  return sgd_launch(false, n, p, g, buf, mask, lr, momentum, weight_decay, grad_scale, first_step, l1_decay, l1_sum,
+                    lr_dev, nullptr, stream);
+}
+
+extern "C" int rcv_sgd_step_det(int64_t n, float* p, const float* g, float* buf, const uint8_t* mask,
+                                float lr, float momentum, float weight_decay, float grad_scale,
+                                int first_step, float l1_decay, double* l1_sum, const float* lr_dev,
+                                void* scratch, uint64_t scratch_bytes, void* stream) {
+  RCV_L1_SCRATCH_CHECK("sgd_step_det");
+  return sgd_launch(true, n, p, g, buf, mask, lr, momentum, weight_decay, grad_scale, first_step, l1_decay, l1_sum,
+                    lr_dev, scratch, stream);
 }
 
 // Stream-ordered memset (a memset node when captured into a CUDA graph: no kernel): the zero fill of the

@@ -67,14 +67,15 @@ __device__ __forceinline__ void load_logits(const float* __restrict__ lp, int64_
   for (int c = 0; c < C; ++c) z[c] = __ldg(lp + (int64_t)c * HW);
 }
 
-// grid: (chunks, N).  One thread per pixel of image blockIdx.y.
-template <int C>
+// grid: (chunks, N).  One thread per pixel of image blockIdx.y.  DET: loss_sums through the ordered flush over det
+// (slot = linear block index) instead of atomics.
+template <int C, bool DET = false>
 __global__ void __launch_bounds__(NT) ce_fwd_kernel(int64_t HW, const float* __restrict__ logits,
                                                      const int64_t* __restrict__ target,
                                                      const float* __restrict__ class_w,
                                                      double* loss_sums, int64_t* argmax_out,
                                                      unsigned long long* conf,
-                                                     unsigned long long* correct) {
+                                                     unsigned long long* correct, void* det) {
   rcv_pdl_enter();
   __shared__ int hist[CMAX * CMAX];
   __shared__ double red[2][NT / 32];
@@ -133,7 +134,10 @@ __global__ void __launch_bounds__(NT) ce_fwd_kernel(int64_t HW, const float* __r
   if (threadIdx.x == 0) {
     double a = 0.0, b = 0.0;
     for (int i = 0; i < NT / 32; ++i) { a += red[0][i]; b += red[1][i]; }
-    if (loss_sums) {
+    if constexpr (DET) {
+      red[0][0] = a;
+      red[0][1] = b;
+    } else if (loss_sums) {
       atomicAdd(loss_sums, a);
       atomicAdd(loss_sums + 1, b);
     }
@@ -142,6 +146,12 @@ __global__ void __launch_bounds__(NT) ce_fwd_kernel(int64_t HW, const float* __r
   if (conf && threadIdx.x < C * C) {
     const int h = hist[threadIdx.x];
     if (h) atomicAdd(conf + (int64_t)n * C * C + threadIdx.x, (unsigned long long)h);
+  }
+  if constexpr (DET) {
+    if (loss_sums) {
+      __syncthreads();
+      rcv_ordered_flush(det, blockIdx.y * gridDim.x + blockIdx.x, gridDim.x * gridDim.y, 2, red[0], loss_sums);
+    }
   }
 }
 
@@ -248,19 +258,52 @@ extern "C" int rcv_maxpool2x2_bwd(int32_t N, int32_t C, int32_t H, int32_t W, co
     default: break;                               \
   }
 
-extern "C" int rcv_ce_fwd(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
-                          const float* class_w, double* loss_sums, int64_t* argmax, int64_t* conf,
-                          int64_t* correct, void* stream) {
+namespace {
+dim3 ce_grid(int32_t N, int64_t HW) {
+  return dim3(blocks_for(HW, rcv_cdiv(148 * 8, N) < 1 ? 1 : rcv_cdiv(148 * 8, N)), N);
+}
+
+int ce_fwd_launch(bool det, int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
+                  const float* class_w, double* loss_sums, int64_t* argmax, int64_t* conf, int64_t* correct,
+                  void* scratch, void* stream) {
   RCV_REQUIRE(N > 0 && HW > 0 && logits && target, RCV_ERR_BAD_ARG, "ce_fwd: bad arg");
   RCV_REQUIRE(C >= 1 && C <= CMAX, RCV_ERR_UNSUPPORTED, "ce_fwd: C=%d (supported 1..8)", C);
   RCV_REQUIRE(N <= 65535, RCV_ERR_UNSUPPORTED, "ce_fwd: N=%d > 65535", N);
-  dim3 grid(blocks_for(HW, rcv_cdiv(148 * 8, N) < 1 ? 1 : rcv_cdiv(148 * 8, N)), N);
+  const dim3 grid = ce_grid(N, HW);
   cudaStream_t st = (cudaStream_t)stream;
-  RCV_CE_DISPATCH(C, (rcv_launch(ce_fwd_kernel<CC>, dim3(grid), dim3(NT), 0, st, HW, logits, target, class_w,
-                                 loss_sums, argmax, reinterpret_cast<unsigned long long*>(conf),
-                                 reinterpret_cast<unsigned long long*>(correct))));
+  unsigned long long* cf = reinterpret_cast<unsigned long long*>(conf);
+  unsigned long long* cr = reinterpret_cast<unsigned long long*>(correct);
+  if (det) {
+    RCV_CE_DISPATCH(C, (rcv_launch(ce_fwd_kernel<CC, true>, grid, dim3(NT), 0, st, HW, logits, target, class_w,
+                                   loss_sums, argmax, cf, cr, scratch)));
+  } else {
+    RCV_CE_DISPATCH(C, (rcv_launch(ce_fwd_kernel<CC>, grid, dim3(NT), 0, st, HW, logits, target, class_w,
+                                   loss_sums, argmax, cf, cr, scratch)));
+  }
   RCV_CHECK_LAUNCH("ce_fwd");
   return RCV_OK;
+}
+}  // namespace
+
+extern "C" int rcv_ce_fwd(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
+                          const float* class_w, double* loss_sums, int64_t* argmax, int64_t* conf,
+                          int64_t* correct, void* stream) {
+  return ce_fwd_launch(false, N, C, HW, logits, target, class_w, loss_sums, argmax, conf, correct, nullptr, stream);
+}
+
+size_t rcv_ce_fwd_det_bytes(int32_t N, int64_t HW) {
+  const dim3 g = ce_grid(N, HW);
+  return rcv_det_bytes((long long)g.x * g.y, 2, sizeof(double));
+}
+
+extern "C" int rcv_ce_fwd_det(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,
+                              const float* class_w, double* loss_sums, int64_t* argmax, int64_t* conf,
+                              int64_t* correct, void* scratch, uint64_t scratch_bytes, void* stream) {
+  RCV_REQUIRE(N > 0 && N <= 65535 && HW > 0, RCV_ERR_BAD_ARG, "ce_fwd_det: bad arg");
+  RCV_REQUIRE(!loss_sums || (scratch && scratch_bytes >= rcv_ce_fwd_det_bytes(N, HW)), RCV_ERR_WORKSPACE,
+              "ce_fwd_det: scratch of %llu bytes, %zu needed", (unsigned long long)scratch_bytes,
+              rcv_ce_fwd_det_bytes(N, HW));
+  return ce_fwd_launch(true, N, C, HW, logits, target, class_w, loss_sums, argmax, conf, correct, scratch, stream);
 }
 
 extern "C" int rcv_ce_bwd(int32_t N, int32_t C, int64_t HW, const float* logits, const int64_t* target,

@@ -13,6 +13,8 @@ gradients are views of one zero-filled flat buffer (or of the caller's arena).
 """
 from __future__ import annotations
 
+import warnings
+
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -497,6 +499,20 @@ class _PlanFn(torch.autograd.Function):
         return (None, None, None, dx, *[gv[id(p)] for p in ctx.plan.params])
 
 
+def _alert_not_deterministic(what: str) -> None:
+    """torch.use_deterministic_algorithms(True): raise RuntimeError naming `what`, or warn under warn_only=True, as
+    torch's own nondeterministic ops do."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{what} does not have a deterministic implementation, but you set "
+           "'torch.use_deterministic_algorithms(True)'. You can turn off determinism just for this operation, or use "
+           "the 'warn_only=True' option.")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg, UserWarning, stacklevel=3)
+    else:
+        raise RuntimeError(msg)
+
+
 def run_plan(plan: Plan, x: torch.Tensor, training: bool) -> Tuple[torch.Tensor, ...]:
     if not x.is_cuda:
         raise RuntimeError(
@@ -504,5 +520,12 @@ def run_plan(plan: Plan, x: torch.Tensor, training: bool) -> Tuple[torch.Tensor,
             "There is no CPU fallback; the CPU oracle under oracle/ is test infrastructure.")
     if x.dtype != torch.float32:
         raise TypeError(f"robocupvision_b200: fp32 input expected, got {x.dtype}")
+    if training:
+        # eval mode sums nothing across CTAs in floating point (the split reduction adds its shares in share order);
+        # train mode adds the BatchNorm batch statistics, and its backward the weight / bias gradients and the
+        # BatchNorm backward sums, with floating-point atomics
+        _alert_not_deterministic(
+            "robocupvision_b200 train-mode forward and backward (BatchNorm batch statistics, weight gradients, "
+            "BatchNorm backward sums)")
     need = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in plan.params))
     return _PlanFn.apply(plan, training, need, x, *plan.params)

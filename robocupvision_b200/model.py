@@ -82,10 +82,30 @@ class _PlanModule(nn.Module):
 
 
 # =============================================================================== losses
+_loss_scratches = {}
+
+
+def _loss_scratch(op, logits):
+    """Under torch.use_deterministic_algorithms(True): scratch for the fixed-order form of the loss reduction (its sums
+    are then bitwise the same run after run on the same device).  Otherwise None: the atomic form.  The backward
+    kernels of both losses are element-wise and need nothing.  One zero-filled scratch per (op, shape, device, stream),
+    allocated on first use and kept: the kernels leave it ready for the next call, and calls on one stream are ordered,
+    so a step in a loop allocates and fills nothing."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return None
+    n, c = logits.shape[0], logits.shape[1]
+    hw = logits.numel() // (n * c)
+    key = (op, n, c, hw, logits.device, torch.cuda.current_stream(logits.device).cuda_stream)
+    scratch = _loss_scratches.get(key)
+    if scratch is None:
+        scratch = _loss_scratches[key] = ops.det_scratch(op, n, c, hw, logits.device)
+    return scratch
+
+
 class _WeightedCE(torch.autograd.Function):
     @staticmethod
     def forward(ctx, logits, target, weight):
-        sums, _, _, _ = ops.ce_fwd(logits, target, weight)
+        sums, _, _, _ = ops.ce_fwd(logits, target, weight, scratch=_loss_scratch(ops.DET_CE_FWD, logits))
         ctx.save_for_backward(logits, target, sums)
         ctx.weight = weight
         return (sums[0] / sums[1]).to(torch.float32)
@@ -98,7 +118,9 @@ class _WeightedCE(torch.autograd.Function):
 
 class CrossEntropyLoss2d(nn.Module):
     """Class-weighted mean of -log softmax(x)[y] over all pixels (model.py:76-82):
-    loss = sum_p w[y_p] * nll_p / sum_p w[y_p].  One fused kernel forward, one backward."""
+    loss = sum_p w[y_p] * nll_p / sum_p w[y_p].  One fused kernel forward, one backward.  Under
+    torch.use_deterministic_algorithms(True) the forward sums in fixed order (rcv_ce_fwd_det): the same logits give
+    bitwise the same loss and gradient, run after run on one device."""
 
     def __init__(self, weight=None):
         super().__init__()
@@ -117,7 +139,7 @@ class CrossEntropyLoss2d(nn.Module):
 class _Dice(torch.autograd.Function):
     @staticmethod
     def forward(ctx, logits, target, weights, eps):
-        sums = ops.dice_fwd(logits, target)
+        sums = ops.dice_fwd(logits, target, scratch=_loss_scratch(ops.DET_DICE_FWD, logits))
         c = logits.shape[1]
         ctx.save_for_backward(logits, target, weights, sums)
         ctx.eps = eps
@@ -133,8 +155,9 @@ class _Dice(torch.autograd.Function):
 class DiceLoss(nn.Module):
     """Optional `--useDice` loss (model.py:5-43): 1 - mean_c(2 w_c I_c / (K_c + eps)) with the soft
     intersection I and cardinality K of softmax(logits) against the one-hot labels, w normalised to sum to C.
-    CUDA logits, 2..8 classes: one fused kernel forward (rcv_dice_fwd) and one backward (rcv_dice_bwd).
-    The single-logit sigmoid form (model.py:25-32, never used by the drivers) stays plain tensor ops."""
+    CUDA logits, 2..8 classes: one fused kernel forward (rcv_dice_fwd) and one backward (rcv_dice_bwd); under
+    torch.use_deterministic_algorithms(True) the forward sums in fixed order (rcv_dice_fwd_det).  The single-logit
+    sigmoid form (model.py:25-32, never used by the drivers) stays plain tensor ops."""
 
     def __init__(self, weights, eps=1e-7):
         super().__init__()

@@ -13,15 +13,16 @@ from typing import Optional, Tuple
 import torch
 
 from . import _lib
-from ._lib import (ENGINE_DIRECT, ENGINE_NARROW, ENGINE_SIMT, ENGINE_UMMA, EPI_AFFINE, EPI_AFFINE_RELU, EPI_NONE,
+from ._lib import (DET_CE_FWD, DET_CE_WEIGHT_SUM, DET_DICE_FWD, DET_L1_SUM, ENGINE_DIRECT, ENGINE_NARROW, ENGINE_SIMT, ENGINE_UMMA, EPI_AFFINE, EPI_AFFINE_RELU, EPI_NONE,
                    EPI_RELU, EPI_RELU_AFFINE, MATH_AUTO, MATH_BF16, MATH_FP32, MATH_TF32, MATH_TF32X3, PACK_DGRAD,
                    PACK_FWD, ConvDesc)
 
 __all__ = [
     "ConvGeom", "conv_fwd", "conv_dgrad", "conv_wgrad", "conv_pack", "conv_packed_bytes", "conv_workspace_bytes", "new_workspace", "conv_takes_partial_residual", "conv_uses_tensor_cores", "conv_engine", "conv_normalises_on_load", "PackTable", "bn_finalize_apply", "PACK_FWD", "PACK_DGRAD", "bn_finalize", "bn_fold", "bn_apply",
     "bn_bwd", "relu_bwd", "channel_sum", "maxpool2x2_fwd", "maxpool2x2_bwd", "maxunpool2x2", "maxunpool2x2_bwd", "upsample_bilinear2x", "upsample_bilinear2x_bwd", "ce_fwd", "ce_bwd",
-    "confusion", "metric_tail", "mask_label_lut", "mask_label_", "label_to_pred", "lp_assemble", "augment", "color_jitter_params", "dice_fwd", "dice_bwd", "adam_l1_step", "sgd_step", "zero_", "zeros", "counter_add", "launch_count", "reset_launch_count",
+    "confusion", "metric_tail", "mask_label_lut", "mask_label_", "label_to_pred", "lp_assemble", "augment", "color_jitter_params", "dice_fwd", "dice_bwd", "adam_l1_step", "sgd_step", "det_scratch_bytes", "det_scratch", "zero_", "zeros", "counter_add", "launch_count", "reset_launch_count",
     "EPI_NONE", "EPI_RELU", "EPI_RELU_AFFINE", "EPI_AFFINE_RELU", "EPI_AFFINE",
+    "DET_CE_FWD", "DET_CE_WEIGHT_SUM", "DET_DICE_FWD", "DET_L1_SUM",
     "MATH_FP32", "MATH_TF32X3", "MATH_AUTO", "MATH_TF32", "MATH_BF16", "ENGINE_SIMT", "ENGINE_DIRECT", "ENGINE_UMMA", "ENGINE_NARROW",
 ]
 
@@ -469,10 +470,15 @@ def head_ce_supported(cin: int, classes: int) -> bool:
     return bool(_lib.load().rcv_head_ce_supported(int(cin), int(classes)))
 
 
-def ce_weight_sum(target, class_w, out, classes: int) -> None:
-    """out[0] += sum over pixels of class_w[target] (the normaliser of the weighted mean loss; labels only)."""
+def ce_weight_sum(target, class_w, out, classes: int, scratch=None) -> None:
+    """out[0] += sum over pixels of class_w[target] (the normaliser of the weighted mean loss; labels only).
+    scratch: det_scratch(DET_CE_WEIGHT_SUM, ...) for the fixed-order sum (rcv_ce_weight_sum_det)."""
     target = _chk(target, torch.int64, "target")
-    _call("rcv_ce_weight_sum", 1, int(classes), target.numel(), _ptr(target), _ptr(class_w), _ptr(out), _stream())
+    if scratch is None:
+        _call("rcv_ce_weight_sum", 1, int(classes), target.numel(), _ptr(target), _ptr(class_w), _ptr(out), _stream())
+    else:
+        _call("rcv_ce_weight_sum_det", 1, int(classes), target.numel(), _ptr(target), _ptr(class_w), _ptr(out),
+              *_scratch_args(scratch), _stream())
 
 
 def head_ce_train(feat, weight, bias, target, class_w, sums, corr, dweight, dbias):
@@ -515,9 +521,10 @@ def concat_channels(a, b) -> torch.Tensor:
 
 # --------------------------------------------------------------------------- loss / metrics
 def ce_fwd(logits, target, class_w=None, want_argmax=False, want_conf=False, want_correct=False, sums=None,
-           corr=None):
+           corr=None, scratch=None):
     """-> (loss_sums float64[2], argmax|None, conf int64[N,C,C]|None, correct int64[1]|None).  sums / corr:
-    caller-zeroed accumulators to use instead of fresh ones."""
+    caller-zeroed accumulators to use instead of fresh ones.  scratch: det_scratch(DET_CE_FWD, ...) for loss sums in
+    fixed order (rcv_ce_fwd_det)."""
     logits = _chk(logits, name="logits")
     target = _chk(target, torch.int64, "target")
     n, c = logits.shape[0], logits.shape[1]
@@ -535,8 +542,12 @@ def ce_fwd(logits, target, class_w=None, want_argmax=False, want_conf=False, wan
         class_w = _chk(class_w, name="class_w")
         if class_w.numel() != c:
             raise ValueError("ce_fwd: class_w must have C entries")
-    _call("rcv_ce_fwd", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(class_w), _ptr(sums), _ptr(am),
-          _ptr(conf), _ptr(corr), _stream())
+    if scratch is None:
+        _call("rcv_ce_fwd", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(class_w), _ptr(sums), _ptr(am),
+              _ptr(conf), _ptr(corr), _stream())
+    else:
+        _call("rcv_ce_fwd_det", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(class_w), _ptr(sums), _ptr(am),
+              _ptr(conf), _ptr(corr), *_scratch_args(scratch), _stream())
     return sums, am, conf, corr
 
 
@@ -659,14 +670,19 @@ def augment(x, params, labels=None, mean=(0.5, 0.0, 0.0), std=(0.5, 0.5, 0.5)):
     return y, lo
 
 
-def dice_fwd(logits, target):
-    """-> float64[2C]: per-class soft intersection and cardinality of softmax(logits) vs the labels."""
+def dice_fwd(logits, target, scratch=None):
+    """-> float64[2C]: per-class soft intersection and cardinality of softmax(logits) vs the labels.  scratch:
+    det_scratch(DET_DICE_FWD, ...) for the fixed-order sums (rcv_dice_fwd_det)."""
     logits = _chk(logits, name="logits")
     target = _chk(target, torch.int64, "target")
     n, c = logits.shape[0], logits.shape[1]
     hw = logits.numel() // (n * c)
     sums = zeros(2 * c, torch.float64, logits.device)
-    _call("rcv_dice_fwd", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(sums), _stream())
+    if scratch is None:
+        _call("rcv_dice_fwd", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(sums), _stream())
+    else:
+        _call("rcv_dice_fwd_det", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(sums), *_scratch_args(scratch),
+              _stream())
     return sums
 
 
@@ -683,17 +699,47 @@ def dice_bwd(logits, target, weights, sums, eps, gscale=None):
 
 
 def adam_l1_step(p, g, m, v, lr, beta1=0.9, beta2=0.999, eps=1e-8, step=1, l1_decay=0.0, grad_scale=1.0,
-                 mask=None, l1_sum=None, step_dev=None, lr_dev=None):
-    _call("rcv_adam_l1_step", 1, p.numel(), _ptr(p), _ptr(g), _ptr(m), _ptr(v), _ptr(mask), float(lr),
-          float(beta1), float(beta2), float(eps), int(step), float(l1_decay), float(grad_scale),
-          _ptr(l1_sum), _ptr(step_dev), _ptr(lr_dev), _stream())
+                 mask=None, l1_sum=None, step_dev=None, lr_dev=None, scratch=None):
+    """scratch: det_scratch(DET_L1_SUM, ...) for l1_sum in fixed order (rcv_adam_l1_step_det)."""
+    args = (p.numel(), _ptr(p), _ptr(g), _ptr(m), _ptr(v), _ptr(mask), float(lr), float(beta1), float(beta2),
+            float(eps), int(step), float(l1_decay), float(grad_scale), _ptr(l1_sum), _ptr(step_dev), _ptr(lr_dev))
+    if scratch is None:
+        _call("rcv_adam_l1_step", 1, *args, _stream())
+    else:
+        _call("rcv_adam_l1_step_det", 1, *args, *_scratch_args(scratch), _stream())
 
 
 def sgd_step(p, g, buf, lr, momentum=0.0, weight_decay=0.0, grad_scale=1.0, mask=None, first_step=False,
-             l1_decay=0.0, l1_sum=None, lr_dev=None):
-    _call("rcv_sgd_step", 1, p.numel(), _ptr(p), _ptr(g), _ptr(buf), _ptr(mask), float(lr), float(momentum),
-          float(weight_decay), float(grad_scale), 1 if first_step else 0, float(l1_decay), _ptr(l1_sum),
-          _ptr(lr_dev), _stream())
+             l1_decay=0.0, l1_sum=None, lr_dev=None, scratch=None):
+    """scratch: det_scratch(DET_L1_SUM, ...) for l1_sum in fixed order (rcv_sgd_step_det)."""
+    args = (p.numel(), _ptr(p), _ptr(g), _ptr(buf), _ptr(mask), float(lr), float(momentum), float(weight_decay),
+            float(grad_scale), 1 if first_step else 0, float(l1_decay), _ptr(l1_sum), _ptr(lr_dev))
+    if scratch is None:
+        _call("rcv_sgd_step", 1, *args, _stream())
+    else:
+        _call("rcv_sgd_step_det", 1, *args, *_scratch_args(scratch), _stream())
+
+
+# --------------------------------------------------------------------------- fixed-order reductions
+def det_scratch_bytes(op: int, n: int, c: int, hw: int) -> int:
+    """Bytes of scratch the fixed-order (_det) form of `op` (DET_CE_FWD, DET_CE_WEIGHT_SUM, DET_DICE_FWD,
+    DET_L1_SUM) needs for N=n, C=c, HW=hw (see rcv_det_scratch_bytes for what each op reads).  Host only."""
+    nb = _lib.load().rcv_det_scratch_bytes(int(op), int(n), int(c), int(hw))
+    if nb == 0:
+        raise ValueError(f"det_scratch_bytes: no fixed-order path for op {op} at N={n}, C={c}, HW={hw}")
+    return nb
+
+
+def det_scratch(op: int, n: int, c: int, hw: int, device) -> torch.Tensor:
+    """Zero-filled scratch for the fixed-order form of `op` (see det_scratch_bytes).  The kernels leave it ready for
+    the next call of the same op and size; one stream at a time."""
+    return zeros(det_scratch_bytes(op, n, c, hw), torch.uint8, device)
+
+
+def _scratch_args(scratch: torch.Tensor):
+    if not scratch.is_cuda or scratch.dtype != torch.uint8 or not scratch.is_contiguous():
+        raise RuntimeError("robocupvision_b200: scratch must be a contiguous CUDA uint8 tensor (det_scratch)")
+    return _ptr(scratch), C.c_uint64(scratch.numel())
 
 
 def zero_(t: torch.Tensor) -> torch.Tensor:
