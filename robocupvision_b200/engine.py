@@ -88,7 +88,8 @@ class Node:
         return hit
 
     def pack_buffer(self, direction: int, math: int, nhw) -> torch.Tensor:
-        """Persistent panel buffer (allocated once per device, math mode and panel size: CUDA-graph safe)."""
+        """Persistent panel buffer (allocated once per device, math mode and panel size; a graph that captured a
+        replaced buffer keeps it alive through Plan.capture_refs)."""
         w = self.conv.weight
         buf = self._pack[direction]
         nbytes = self._pack_bytes.get((direction, math, nhw))
@@ -204,6 +205,16 @@ class Plan:
         if ws is None or ws.device != dev or ws.numel() < need:
             ws = self._workspace = ops.new_workspace(need, dev)
         return ws
+
+    def capture_refs(self) -> List[torch.Tensor]:
+        """The device buffers a CUDA graph captured now can bake in: the conv workspace, every node's weight panels and
+        the device table of every cached PackTable.  The plan replaces them when an input size needs a larger or a
+        different buffer, so whoever keeps a graph keeps this list beside it: a replaced buffer is then freed only
+        once no graph that uses it is left."""
+        refs = [] if self._workspace is None else [self._workspace]
+        refs += [b for nd in self.nodes for b in nd._pack if b is not None]
+        refs += [tbl.table for tbl in self._pack_tables.values()]
+        return refs
 
     def _ensure_packed(self, directions, fresh: bool, x_requires_grad: bool, nhw):
         """Weight panels of every tensor-core layer, re-packed in ONE launch when `fresh` (training:

@@ -219,6 +219,7 @@ class TrainStep:
         self.correct = None
         self.use_graph = use_graph
         self.graph = None
+        self._graph_refs = []  # the plan's buffers self.graph bakes in (Plan.capture_refs): freed with the graph
         self.static_x = None
         self.static_y = None
         self.kernels_per_step = 0
@@ -416,6 +417,7 @@ class TrainStep:
         with torch.cuda.graph(g):
             self.loss_sums, self.l1_sum, self.correct = self._step_impl(self.static_x, self.static_y)
         self.graph = g
+        self._graph_refs = self.plan.capture_refs()
         self._pipe = None  # the staging slots have the old shape
         g.replay()
 
@@ -574,7 +576,10 @@ class EvalStep:
             with torch.cuda.graph(g):
                 out = self._eager(sx, sy)
             self.kernels_per_call = ops.launch_count() - k0  # rcv_* kernels one replay launches
-            ent = {"graph": g, "sx": sx, "sy": sy, "out": out, "state": self._state_key()}
+            plan = self.model._get_plan() if hasattr(self.model, "_get_plan") else None
+            # the plan's buffers the graph bakes in stay alive while the graph does, whatever sizes run in between
+            refs = plan.capture_refs() if plan is not None else []
+            ent = {"graph": g, "sx": sx, "sy": sy, "out": out, "state": self._state_key(), "refs": refs}
             self._graphs[key] = ent
         ent["sx"].copy_(x, non_blocking=True)
         ent["sy"].copy_(y, non_blocking=True)

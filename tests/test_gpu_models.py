@@ -13,10 +13,9 @@ import synth
 from nets import ROBO_VARIANTS, pb_fcn_state, robo_state
 from oracle import ref_metrics, ref_model as R
 from oracle.ref_train import OracleTrainer
-from util import assert_close, load_ckpt, load_golden, with_nbt
+from util import LOGIT_TOL, assert_close, check_eval_outputs, load_ckpt, load_golden, with_nbt
 
 pytestmark = pytest.mark.gpu
-LOGIT_TOL = 1e-4
 
 
 def _check_eval(tag, model, oracle_fwd, golden, num_classes=5, weights=synth.CLASS_WEIGHTS):
@@ -30,31 +29,18 @@ def _check_eval(tag, model, oracle_fwd, golden, num_classes=5, weights=synth.CLA
         out = ev(x.cuda(), y.cuda())
         with torch.no_grad():
             ref = oracle_fwd(x)
-        logits = out["logits"].cpu()
-        err = assert_close(f"{tag} logits[{i}]", logits, ref, LOGIT_TOL)
+        # oracle logits; the reference's own label maps and loss
+        am_ref = torch.from_numpy(golden[f"argmax{i}"].astype(np.int64))
+        err, flips = check_eval_outputs(f"{tag}[{i}]", out, ref, am_ref, y, float(golden[f"loss{i}"]), num_classes)
         # golden (reference-produced) subsample
-        lf = logits.reshape(-1)
+        lf = out["logits"].cpu().reshape(-1)
         sub = lf[::13] if lf.numel() > 50000 else lf
         gsub = torch.from_numpy(golden[f"logits_sub{i}"])
         assert_close(f"{tag} golden logits[{i}]", sub, gsub, LOGIT_TOL)
-        # argmax: exact outside near-ties
-        top2 = ref.topk(2, dim=1).values
-        margin = top2[:, 0] - top2[:, 1]
-        am = out["argmax"].cpu()
-        am_ref = torch.from_numpy(golden[f"argmax{i}"].astype(np.int64))
-        diff = am != am_ref
-        assert not bool((diff & (margin >= 1e-4)).any()), f"{tag}: argmax differs outside near-ties"
-        if not bool(diff.any()):
+        if flips == 0:
             assert (out["conf"].cpu().numpy() == golden[f"conf{i}"]).all(), f"{tag}: confusion counts"
-        conf_own = ref_metrics.confusion_per_image(am.numpy(), y.numpy(), num_classes)
-        assert (out["conf"].cpu().numpy() == conf_own).all(), f"{tag}: confusion vs own label map"
-        assert int(out["correct"]) == int((am == y).sum())
-        iou_ref = ref_metrics.iou_sums(conf_own)
-        assert np.allclose(out["iou_sum"].cpu().numpy(), iou_ref, rtol=0, atol=1e-12)
-        gl = float(golden[f"loss{i}"])
-        assert abs(float(out["loss"]) - gl) <= 1e-5 * max(1.0, abs(gl)), f"{tag}: loss {float(out['loss'])} vs {gl}"
         print(f"{tag}[{i}] {n}x{c}x{h}x{w}: logits err {err:.2e} (absmax {float(golden[f'logits_absmax{i}']):.1f}), "
-              f"argmax flips {int(diff.sum())}, min margin {float(golden[f'margin_min{i}']):.2e}")
+              f"argmax flips {flips}, min margin {float(golden[f'margin_min{i}']):.2e}")
         i += 1
     assert i > 0
 

@@ -407,6 +407,76 @@ def test_engine_backward_side_stream_code_path_on_cpu(cpu_engine, monkeypatch):
     assert waits.count(("wait", True, False)) == 1 and waits[-1] == ("wait", True, False)   # one join, at the end
 
 
+def test_graph_owner_keeps_the_plan_buffers_its_capture_baked_in(cpu_engine, monkeypatch):
+    """EvalStep(use_graph=True) at batch 4, then 8, on the engine with size-dependent stand-ins for the workspace and
+    panel sizes (every conv a tensor-core layer) and torch.cuda's graph and stream objects replaced by inert ones:
+    the second size makes Plan.workspace return a larger buffer and replaces every panel and the pack table.  The
+    tensors Plan.capture_refs returned before are then still referenced through the EvalStep, and freed once it is
+    dropped."""
+    import contextlib
+    import gc
+    import weakref
+
+    from robocupvision_b200 import train
+    from util import tensors_held_by
+    engine, fake = cpu_engine
+
+    class PackTable:
+        def __init__(self, jobs, math=None, sizes=None):
+            self.table = torch.zeros(64 * len(jobs), dtype=torch.uint8)
+
+        def run(self):
+            pass
+
+    class Stream:
+        def __init__(self, device=None):
+            pass
+
+        def wait_stream(self, other):
+            pass
+
+    class Graph:
+        def replay(self):
+            pass
+
+    monkeypatch.setattr(fake, "conv_uses_tensor_cores", lambda g, direction, math=None: True)
+    monkeypatch.setattr(fake, "conv_workspace_bytes", lambda g, n, h, w, direction=0, math=None: 4096 * n * h * w // 3072)
+    monkeypatch.setattr(fake, "new_workspace", lambda nbytes, dev: torch.zeros(max(nbytes, 1024), dtype=torch.uint8))
+    monkeypatch.setattr(fake, "conv_packed_bytes",
+                        lambda g, direction, math=None, nhw=None: 4 * g.cin * g.cout * g.k * g.k + 256 * nhw[0])
+    monkeypatch.setattr(fake, "PackTable", PackTable)
+    monkeypatch.setattr(torch.cuda, "current_stream", lambda device=None: Stream())
+    monkeypatch.setattr(torch.cuda, "Stream", Stream)
+    monkeypatch.setattr(torch.cuda, "stream", lambda s: contextlib.nullcontext())
+    monkeypatch.setattr(torch.cuda, "synchronize", lambda device=None: None)
+    monkeypatch.setattr(torch.cuda, "CUDAGraph", Graph)
+    monkeypatch.setattr(torch.cuda, "graph", lambda g: contextlib.nullcontext())
+    monkeypatch.setattr(train.EvalStep, "_eager",
+                        lambda self, x, y: {"logits": self.model._get_plan().forward(x, training=False, save=False)[0][0]})
+    make, _, cin = _cases()["robo_default"]
+    torch.manual_seed(12345678)
+    m = make().eval()
+    plan = m._get_plan()
+    es = train.EvalStep(m, use_graph=True)
+    with torch.no_grad():
+        es(synth.images(4, cin, 48, 64, seed=1), synth.labels_random(4, 48, 64))
+        ws4 = plan.workspace((4, 48, 64), torch.device("cpu"))
+        refs = plan.capture_refs()
+        assert any(t is ws4 for t in refs)
+        assert len(refs) == 1 + sum(1 for nd in plan.nodes if nd.kind == "conv") + len(plan._pack_tables)
+        es(synth.images(8, cin, 48, 64, seed=2), synth.labels_random(8, 48, 64))
+        ws8 = plan.workspace((8, 48, 64), torch.device("cpu"))
+    assert ws8 is not ws4 and ws8.numel() > ws4.numel()
+    # every buffer of the first capture was replaced: the plan holds none of them, the EvalStep holds all of them
+    assert not {id(t) for t in refs} & {id(t) for t in plan.capture_refs()}
+    held = tensors_held_by(es)
+    assert all(id(t) in held for t in refs), "the EvalStep must hold every buffer its graphs baked in"
+    dead = [weakref.ref(t) for t in refs]
+    del refs, ws4, es
+    gc.collect()
+    assert all(r() is None for r in dead), "dropping the graph's owner must free the buffers only its graph used"
+
+
 @pytest.mark.parametrize("tag", ["robo_default", "labelprop"])
 def test_fused_head_wiring_on_cpu(tag, cpu_engine):
     """TrainStep's fused classifier head: Plan.forward(stop_before=head) + ops.head_ce_train + Plan.backward(seed=...)
