@@ -353,6 +353,33 @@ int rcv_head_ce_train(int32_t N, int32_t Cin, int32_t C, int64_t HW, const float
                       double* loss_sums, int64_t* correct, float* dfeat, float* dweight, float* dbias,
                       void* stream);
 
+/* ---- classifier head of a Dice-loss training step, two passes ------------ */
+/* The 1x1 classifier conv, DiceLoss (model.py:5-43, the --useDice option), the argmax / correct-pixel count and their
+ * backward in TWO passes over the decoder's last feature map (the Dice gradient of every pixel depends on the
+ * batch-wide sums, so one pass cannot do it).  Replaces, inside TrainStep(loss="dice"), the sequence rcv_conv_fwd
+ * (head) -> rcv_dice_fwd -> rcv_dice_bwd -> rcv_conv_dgrad + rcv_conv_wgrad (head); the logits and their gradient
+ * never exist in memory.  Shapes as rcv_head_ce_train: feat, dfeat [N,Cin,HW]; weight, dweight [C,Cin]; bias, dbias
+ * [C] or NULL; target int64 [N,HW].  Pixels labelled outside [0,C) contribute nothing, to the sums or to the
+ * gradient (rcv_dice_fwd adds their softmax to the cardinality).  Supported: what rcv_head_ce_supported accepts (2..8
+ * classes over 8 or 16 channels); anything else RCV_ERR_UNSUPPORTED.
+ * Pass 1, rcv_head_dice_fwd: logits = weight feat + bias; sums (double[2*C], caller zeroes) as rcv_dice_fwd:
+ * sums[c] += sum_p softmax_c(p)*[y_p==c], sums[C+c] += sum_p (softmax_c(p) + [y_p==c]); correct (int64[1] or NULL)
+ * += #(argmax == y), lowest class index among equal maxima. */
+int rcv_head_dice_fwd(int32_t N, int32_t Cin, int32_t C, int64_t HW, const float* feat, const float* weight,
+                      const float* bias, const int64_t* target, double* sums, int64_t* correct, void* stream);
+/* Pass 2, rcv_head_dice_train, after pass 1 on the same stream: with the finished sums, a_c = 2 w_c / (C (K_c+eps)),
+ * b_c = 2 w_c I_c / (C (K_c+eps)^2) (I_c = sums[c], K_c = sums[C+c]), g_c = -a_c [y==c] + b_c and
+ * dlogits_j = gscale p_j (g_j - sum_c p_c g_c), exactly rcv_dice_bwd's arithmetic; dfeat = weight^T dlogits (written);
+ * dweight += dlogits feat^T; dbias += dlogits.  weights: the normalised w (device float[C], w = weights/sum*C on the
+ * host as DiceLoss does; NULL = 1); gscale device float or NULL (1).  loss (double[2] or NULL) = [1 - mean_c(2 w_c
+ * I_c / (K_c+eps)), 1.0]: a numerator / denominator pair, so readers of the CE loss sums read it unchanged. */
+int rcv_head_dice_train(int32_t N, int32_t Cin, int32_t C, int64_t HW, const float* feat, const float* weight,
+                        const float* bias, const int64_t* target, const float* weights, const double* sums, float eps,
+                        const float* gscale, double* loss, float* dfeat, float* dweight, float* dbias, void* stream);
+/* loss (double[2]) = [1 - mean_c(2 w_c sums[c] / (sums[C+c] + eps)), 1.0] from the sums of rcv_dice_fwd: the loss
+ * cell of rcv_head_dice_train for the unfused Dice step, one single-thread launch.  weights as above, C = 2..8. */
+int rcv_dice_loss(int32_t C, const double* sums, const float* weights, float eps, double* loss, void* stream);
+
 /* dst[n, dst_offset + c, :] = src[n, src_offset + c, :] for c < count; src [N,src_channels,HW], dst
  * [N,dst_channels,HW].  The channel moves of the skip wiring that no producer can fold: ROBO_UNet --v2's
  * torch.cat([layer(up), downs[-(i+2)]], 1) (model.py:507; two calls fill the concatenated tensor), the gradient

@@ -91,6 +91,9 @@ SIGNATURES = {
     "rcv_head_ce_supported": [_i32, _i32],
     "rcv_ce_weight_sum": [_i32, _i64, _p, _p, _p, _p],
     "rcv_head_ce_train": [_i32, _i32, _i32, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
+    "rcv_head_dice_fwd": [_i32, _i32, _i32, _i64, _p, _p, _p, _p, _p, _p, _p],
+    "rcv_head_dice_train": [_i32, _i32, _i32, _i64, _p, _p, _p, _p, _p, _p, _f32, _p, _p, _p, _p, _p, _p],
+    "rcv_dice_loss": [_i32, _p, _p, _f32, _p, _p],
     "rcv_peer_flag_bytes": [],
     "rcv_peer_alloc": [C.c_uint64, C.POINTER(C.c_void_p), _p],
     "rcv_peer_open": [_p, C.POINTER(C.c_void_p)],

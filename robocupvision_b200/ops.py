@@ -20,7 +20,7 @@ from ._lib import (DET_CE_FWD, DET_CE_WEIGHT_SUM, DET_DICE_FWD, DET_L1_SUM, ENGI
 __all__ = [
     "ConvGeom", "conv_fwd", "conv_dgrad", "conv_wgrad", "conv_pack", "conv_packed_bytes", "conv_workspace_bytes", "new_workspace", "conv_takes_partial_residual", "conv_uses_tensor_cores", "conv_engine", "conv_normalises_on_load", "PackTable", "bn_finalize_apply", "PACK_FWD", "PACK_DGRAD", "bn_finalize", "bn_fold", "bn_apply",
     "bn_bwd", "relu_bwd", "channel_sum", "maxpool2x2_fwd", "maxpool2x2_bwd", "maxunpool2x2", "maxunpool2x2_bwd", "upsample_bilinear2x", "upsample_bilinear2x_bwd", "ce_fwd", "ce_bwd",
-    "confusion", "metric_tail", "mask_label_lut", "mask_label_", "label_to_pred", "lp_assemble", "augment", "color_jitter_params", "dice_fwd", "dice_bwd", "adam_l1_step", "sgd_step", "det_scratch_bytes", "det_scratch", "zero_", "zeros", "counter_add", "launch_count", "reset_launch_count",
+    "confusion", "metric_tail", "mask_label_lut", "mask_label_", "label_to_pred", "lp_assemble", "augment", "color_jitter_params", "dice_fwd", "dice_bwd", "dice_loss", "head_dice_fwd", "head_dice_train", "adam_l1_step", "sgd_step", "det_scratch_bytes", "det_scratch", "zero_", "zeros", "counter_add", "launch_count", "reset_launch_count",
     "EPI_NONE", "EPI_RELU", "EPI_RELU_AFFINE", "EPI_AFFINE_RELU", "EPI_AFFINE",
     "DET_CE_FWD", "DET_CE_WEIGHT_SUM", "DET_DICE_FWD", "DET_L1_SUM",
     "MATH_FP32", "MATH_TF32X3", "MATH_AUTO", "MATH_TF32", "MATH_BF16", "ENGINE_SIMT", "ENGINE_DIRECT", "ENGINE_UMMA", "ENGINE_NARROW",
@@ -496,6 +496,44 @@ def head_ce_train(feat, weight, bias, target, class_w, sums, corr, dweight, dbia
     return dfeat
 
 
+def _head_shapes(fn, feat, weight, target):
+    n, cin, h, w_ = feat.shape
+    c = weight.shape[0]
+    if weight.numel() != c * cin or tuple(target.shape) != (n, h, w_):
+        raise ValueError(f"{fn}: feat {tuple(feat.shape)}, weight {tuple(weight.shape)}, target {tuple(target.shape)}")
+    return n, cin, c, h * w_
+
+
+def head_dice_fwd(feat, weight, bias, target, sums, corr) -> None:
+    """Pass 1 of the Dice-loss classifier head (rcv_head_dice_fwd): sums float64[2C] += the soft intersection and
+    cardinality of softmax(weight feat + bias) against the labels; corr int64[1] (or None) += correct pixels."""
+    feat = _chk(feat, name="feat")
+    target = _chk(target, torch.int64, "target")
+    n, cin, c, hw = _head_shapes("head_dice_fwd", feat, weight, target)
+    _call("rcv_head_dice_fwd", 1, n, cin, c, hw, _ptr(feat), _ptr(weight), _ptr(bias), _ptr(target), _ptr(sums),
+          _ptr(corr), _stream())
+
+
+def head_dice_train(feat, weight, bias, target, weights, sums, eps, loss, dweight, dbias, gscale=None):
+    """Pass 2 of the Dice-loss classifier head (rcv_head_dice_train), after head_dice_fwd filled `sums`: -> dfeat.
+    weights: the normalised Dice weights float32[C] (or None); loss: float64[2] (or None) <- [dice loss, 1.0];
+    dweight, dbias are accumulated into."""
+    feat = _chk(feat, name="feat")
+    target = _chk(target, torch.int64, "target")
+    n, cin, c, hw = _head_shapes("head_dice_train", feat, weight, target)
+    if gscale is not None:
+        gscale = _chk(gscale.reshape(1).to(torch.float32), name="gscale")
+    dfeat = torch.empty_like(feat)
+    _call("rcv_head_dice_train", 1, n, cin, c, hw, _ptr(feat), _ptr(weight), _ptr(bias), _ptr(target), _ptr(weights),
+          _ptr(sums), float(eps), _ptr(gscale), _ptr(loss), _ptr(dfeat), _ptr(dweight), _ptr(dbias), _stream())
+    return dfeat
+
+
+def dice_loss(sums, weights, eps, loss) -> None:
+    """loss float64[2] <- [1 - mean_c(2 w_c I_c / (K_c + eps)), 1.0] from dice_fwd's sums (rcv_dice_loss)."""
+    _call("rcv_dice_loss", 1, sums.numel() // 2, _ptr(sums), _ptr(weights), float(eps), _ptr(loss), _stream())
+
+
 def channel_slice(x, offset: int, count: int) -> torch.Tensor:
     """x[:, offset:offset+count] as a dense tensor (the gradient halves of a concatenated skip, the gradient of
     LabelProp's partial skip)."""
@@ -670,14 +708,16 @@ def augment(x, params, labels=None, mean=(0.5, 0.0, 0.0), std=(0.5, 0.5, 0.5)):
     return y, lo
 
 
-def dice_fwd(logits, target, scratch=None):
+def dice_fwd(logits, target, scratch=None, sums=None):
     """-> float64[2C]: per-class soft intersection and cardinality of softmax(logits) vs the labels.  scratch:
-    det_scratch(DET_DICE_FWD, ...) for the fixed-order sums (rcv_dice_fwd_det)."""
+    det_scratch(DET_DICE_FWD, ...) for the fixed-order sums (rcv_dice_fwd_det).  sums: a caller-zeroed float64[2C] to
+    accumulate into instead of a fresh one."""
     logits = _chk(logits, name="logits")
     target = _chk(target, torch.int64, "target")
     n, c = logits.shape[0], logits.shape[1]
     hw = logits.numel() // (n * c)
-    sums = zeros(2 * c, torch.float64, logits.device)
+    if sums is None:
+        sums = zeros(2 * c, torch.float64, logits.device)
     if scratch is None:
         _call("rcv_dice_fwd", 1, n, c, hw, _ptr(logits), _ptr(target), _ptr(sums), _stream())
     else:

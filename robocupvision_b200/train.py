@@ -88,7 +88,7 @@ class TrainStep:
                  weight_decay: float = 0.0, lr_mults: Optional[Sequence] = None,
                  process_group=None, use_graph: bool = True, overlap_comm: bool = True, n_buckets: int = 3,
                  force_comm_path: bool = False, reduce: Optional[str] = None,
-                 fused_head: bool = _FUSED_HEAD):
+                 fused_head: bool = _FUSED_HEAD, loss: str = "ce", dice_eps: float = 1e-7):
         """masks: pruneModelNew-style list of bool tensors for the >1-D parameters, in parameter
         order (train.py:59-65); with masks the L1 term is dropped (train.py:53).
         optimizer: "adam" (train.py:357-363; torch defaults, no weight decay) or "sgd" (trainer.py:182-184:
@@ -104,8 +104,18 @@ class TrainStep:
         fused_head: run the classifier conv, the loss, the argmax and their backward as one kernel
         (ops.head_ce_train) where the plan ends in a bare 1x1 conv of 2..8 classes over 8 or 16 channels;
         otherwise (and with RCV_B200_FUSED_HEAD=0) the separate kernels run.
+        loss: "ce" (CrossEntropyLoss2d, class_weights its weights) or "dice" (the reference's --useDice:
+        DiceLoss(class_weights, dice_eps), the weights normalised to sum to the class count as DiceLoss does, all ones
+        without class_weights).  Under "dice" the fused head is two kernels (ops.head_dice_fwd: the batch-wide sums
+        and the correct count; ops.head_dice_train: the backward), the unfused head runs dice_fwd / dice_bwd on the
+        logits.  The raw sums [intersection (C) | cardinality (C)] are kept in `dice_sums`, and the loss sums hold
+        [dice loss, 1.0], so step(), loss_value() and step_async() read the Dice loss unchanged.  With N ranks the
+        sums are rank-local and the gradients averaged: each rank's loss is the Dice loss of its own shard, the
+        semantics DistributedDataParallel gives the reference's loop.
         The optimiser passes of the buckets run on the side stream with one rank too (overlap_comm): they overlap the
         encoder's backward (+0.5 % on the single-GPU step)."""
+        if loss not in ("ce", "dice"):
+            raise ValueError(f"TrainStep: loss must be 'ce' or 'dice', got {loss!r}")
         if optimizer not in ("adam", "sgd"):
             raise ValueError(f"TrainStep: optimizer must be 'adam' or 'sgd', got {optimizer!r}")
         if optimizer == "adam" and (weight_decay != 0.0 or momentum != 0.0):
@@ -167,6 +177,16 @@ class TrainStep:
                 if p.dim() > 1:
                     self.mask[o:o + k] = masks[i].reshape(-1).to(dev).to(torch.uint8)
                     i += 1
+        self.loss = loss
+        self.dice_eps = float(dice_eps)
+        if loss == "dice":
+            if len(self.plan.outputs) != 1 or self.plan.nodes[self.plan.outputs[0] - 1].kind != "conv":
+                raise ValueError("TrainStep(loss='dice'): the plan must end in one classifier conv")
+            ncls = self.plan.nodes[self.plan.outputs[0] - 1].geom.cout
+            w = torch.ones(ncls) if class_weights is None else torch.as_tensor(class_weights, dtype=torch.float32)
+            if w.numel() != ncls:
+                raise ValueError(f"TrainStep(loss='dice'): {w.numel()} class weights for {ncls} classes")
+            class_weights = w / w.sum().item() * w.shape[0]  # DiceLoss.__init__
         self.class_w = None if class_weights is None else torch.as_tensor(
             class_weights, dtype=torch.float32).to(dev)
         # lr groups: contiguous arena ranges (padding included) with a multiplier
@@ -200,18 +220,24 @@ class TrainStep:
         self.step_dev = _zeros(1, torch.int32, dev)
         # every small accumulator of a step in ONE buffer (one memset per step):
         # [l1 sum | CE loss sums (2) | correct pixels (int64 view) | BN batch statistics | BN backward sums]
+        # loss="dice" appends [Dice sums (2C) | the unused loss sums of the correct-count pass of the unfused head (2)]
+        # and keeps [dice loss, 1.0] where the CE loss sums are
         ns = self.plan.n_stats
-        self._accum = _zeros(4 + 2 * ns, torch.float64, dev)
+        ndice = 2 * self.class_w.numel() + 2 if loss == "dice" else 0
+        self._accum = _zeros(4 + 2 * ns + ndice, torch.float64, dev)
         self._acc_l1, self._acc_ce = self._accum[0:1], self._accum[1:3]
         self._acc_corr = self._accum[3:4].view(torch.int64)
         self._acc_stats, self._acc_sums = self._accum[4:4 + ns], self._accum[4 + ns:4 + 2 * ns]
+        self.dice_sums = self._accum[4 + 2 * ns:4 + 2 * ns + ndice - 2] if loss == "dice" else None
+        self._acc_spare = self._accum[4 + 2 * ns + ndice - 2:] if loss == "dice" else None
         # distributed
         self.comm_path = overlap_comm or force_comm_path
         self.comm_stream = torch.cuda.Stream(device=dev) if self.comm_path else None
         # (first plan node, arena start, arena end), in the order backward completes them (arena tail first)
         self.buckets = dp.plan_buckets([[self.offsets[id(p)] for p in nd.params()] for nd in self.plan.nodes],
                                        [(o, k) for _, o, k in self.table], n, n_buckets) if self.comm_path else []
-        # the classifier head in one pass (ops.head_ce_train) where the plan ends in a bare 1x1 conv the kernel covers
+        # the classifier head in one pass (ops.head_ce_train; two for Dice) where the plan ends in a bare 1x1 conv the
+        # kernel covers
         self._head = self.plan.fusable_head() if fused_head else -1
         # outputs (device scalars)
         self.loss_sums = None
@@ -288,7 +314,7 @@ class TrainStep:
         ops.counter_add(self.step_dev, 1)
         head = self._head
         seed = None
-        if head >= 0:
+        if head >= 0 and self.loss == "ce":
             # the normaliser of the weighted mean loss depends on the labels only: produced here, so that the head
             # needs ONE pass (classifier conv + loss + argmax + their backward, ops.head_ce_train)
             ops.ce_weight_sum(y, self.class_w, self._acc_ce[1:2], self.plan.nodes[head].geom.cout)
@@ -296,9 +322,11 @@ class TrainStep:
                                         stop_before=head if head >= 0 else None)
         if head >= 0 and saved[2].get(self.plan.nodes[head].src) is not None:
             raise RuntimeError("TrainStep: the classifier reads a BatchNorm that was deferred to its consumer")
-        if head >= 0:
+        sums, corr = self._acc_ce, self._acc_corr
+        if self.loss == "dice":
+            seed, gouts = self._dice_head(outs, saved, y)
+        elif head >= 0:
             nd = self.plan.nodes[head]
-            sums, corr = self._acc_ce, self._acc_corr
             dfeat = ops.head_ce_train(saved[0][nd.src], nd.conv.weight.detach(),
                                       None if nd.conv.bias is None else nd.conv.bias.detach(), y, self.class_w, sums,
                                       corr, self.grad_views[id(nd.conv.weight)],
@@ -336,11 +364,30 @@ class TrainStep:
         self.kernels_per_step = ops.launch_count() - k0
         return sums, l1, corr
 
+    def _dice_head(self, outs, saved, y):
+        """The Dice loss, its gradient seed for Plan.backward and the correct count: (seed, gouts)."""
+        eps, w = self.dice_eps, self.class_w
+        if self._head >= 0:
+            nd = self.plan.nodes[self._head]
+            feat, wt = saved[0][nd.src], nd.conv.weight.detach()
+            bias = None if nd.conv.bias is None else nd.conv.bias.detach()
+            ops.head_dice_fwd(feat, wt, bias, y, self.dice_sums, self._acc_corr)
+            dfeat = ops.head_dice_train(feat, wt, bias, y, w, self.dice_sums, eps, self._acc_ce,
+                                        self.grad_views[id(nd.conv.weight)],
+                                        None if nd.conv.bias is None else self.grad_views[id(nd.conv.bias)])
+            return {nd.src: dfeat}, [None]
+        logits = outs[0]
+        ops.dice_fwd(logits, y, sums=self.dice_sums)
+        ops.ce_fwd(logits, y, None, want_correct=True, sums=self._acc_spare, corr=self._acc_corr)
+        ops.dice_loss(self.dice_sums, w, eps, self._acc_ce)
+        return None, [ops.dice_bwd(logits, y, w, self.dice_sums, eps)]
+
     def step(self, x: torch.Tensor, y: torch.Tensor):
         """One training step on x [B,Cin,H,W] fp32, y [B,H,W] int64 (device tensors, or pinned
         host tensors which are copied H2D straight into the step's static input buffers).
         Returns (loss_sums float64[2], l1_sum float64[1], correct int64[1]) device tensors:
-        CE loss = loss_sums[0]/loss_sums[1]; total = CE + l1_decay*l1_sum."""
+        CE loss = loss_sums[0]/loss_sums[1] (the Dice loss under loss="dice", loss_sums[1] = 1);
+        total = CE + l1_decay*l1_sum."""
         self.model.train()
         self.plan.epoch += 1  # parameters / BN buffers change under raw kernels (also on graph replay)
         if not self.use_graph:
