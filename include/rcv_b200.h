@@ -255,6 +255,15 @@ int rcv_bn_finalize_apply(int32_t N, int32_t C, int64_t HW, const double* stats,
                           int relu, const float* residual, int32_t res_channels, float* y, float* scale,
                           float* shift, float* save_mean, float* save_invstd,
                           int64_t* num_batches_tracked, void* stream);
+/* The same with the element count per channel of the statistics given: count = N*HW gives rcv_bn_finalize_apply;
+ * a global batch over ranks passes N*HW*world for statistics summed over the ranks.  The running-variance update
+ * uses count/(count-1). */
+int rcv_bn_finalize_apply_count(int32_t N, int32_t C, int64_t HW, int64_t count, const double* stats,
+                                const float* gamma, const float* beta, float* running_mean,
+                                float* running_var, float momentum, float eps, const float* z,
+                                int relu, const float* residual, int32_t res_channels, float* y, float* scale,
+                                float* shift, float* save_mean, float* save_invstd,
+                                int64_t* num_batches_tracked, void* stream);
 
 /* Backward of y = act(scale*z+shift) composed with the producer's own ReLU.
  * order = RCV_EPI_RELU_AFFINE: z = relu(conv), y = bn(z)      (model.py:116)
@@ -560,6 +569,18 @@ int rcv_peer_free(void* ptr);    /* a pointer rcv_peer_alloc returned */
  * world = 1 is legal (flags and barriers run, the sums are the gradients themselves). */
 int rcv_peer_allreduce(int32_t world, int32_t rank, int32_t slot, float* const* arenas, uint32_t* const* flags,
                        int64_t offset, int64_t count, int32_t* status, void* stream);
+
+/* Small-vector exchange (global-batch BatchNorm statistics and backward sums, loss normalisers, correct counts):
+ * bufs[rank][offset, offset+count) <- scale * sum over ranks of bufs[q][offset, offset+count), added in rank order (the
+ * same bits on every rank).  ONE CTA per launch: a ready barrier, every rank loads all N copies, a done barrier ("I
+ * have read yours"), then each rank writes only its OWN buffer, in place.  bufs: HOST array of device pointers in rank
+ * order (peer-mapped, own buffer included), flags as for rcv_peer_allreduce.  offset, count: elements; count <= 4096.
+ * Use a slot no concurrent rcv_peer_allreduce uses.  Same status / time-out rules as rcv_peer_allreduce. */
+int rcv_peer_allreduce_f64(int32_t world, int32_t rank, int32_t slot, double* const* bufs, uint32_t* const* flags,
+                           int64_t offset, int64_t count, double scale, int32_t* status, void* stream);
+/* int64 form (exact sums, no scale): the correct-pixel count */
+int rcv_peer_allreduce_i64(int32_t world, int32_t rank, int32_t slot, int64_t* const* bufs, uint32_t* const* flags,
+                           int64_t offset, int64_t count, int32_t* status, void* stream);
 
 #ifdef __cplusplus
 }

@@ -75,6 +75,8 @@ SIGNATURES = {
     "rcv_bn_apply": [_i32, _i32, _i64, _p, _p, _p, C.c_int, _p, _i32, _p, _p],
     "rcv_bn_finalize_apply": [_i32, _i32, _i64, _p, _p, _p, _p, _p, _f32, _f32, _p, C.c_int, _p, _i32, _p, _p, _p, _p,
                               _p, _p, _p],
+    "rcv_bn_finalize_apply_count": [_i32, _i32, _i64, _i64, _p, _p, _p, _p, _p, _f32, _f32, _p, C.c_int, _p, _i32, _p,
+                                    _p, _p, _p, _p, _p, _p],
     "rcv_bn_bwd_reduce": [_i32, _i32, _i64, C.c_int, _p, _p, _p, _p, _p, _p, _p, _p],
     "rcv_bn_bwd_apply": [_i32, _i32, _i64, C.c_int, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "rcv_bn_bwd_is_fused": [_i32, _i32, _i64],
@@ -100,6 +102,9 @@ SIGNATURES = {
     "rcv_peer_close": [_p],
     "rcv_peer_free": [_p],
     "rcv_peer_allreduce": [_i32, _i32, _i32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i64, _i64, _p, _p],
+    "rcv_peer_allreduce_f64": [_i32, _i32, _i32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i64, _i64, C.c_double,
+                               _p, _p],
+    "rcv_peer_allreduce_i64": [_i32, _i32, _i32, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i64, _i64, _p, _p],
     "rcv_ce_fwd": [_i32, _i32, _i64, _p, _p, _p, _p, _p, _p, _p, _p],
     "rcv_ce_bwd": [_i32, _i32, _i64, _p, _p, _p, _p, _p, _p, _p],
     "rcv_confusion": [_i32, _i32, _i64, _p, _p, _p, _p],

@@ -579,17 +579,19 @@ extern "C" int rcv_bn_apply(int32_t N, int32_t C, int64_t HW, const float* z, co
   return RCV_OK;
 }
 
-extern "C" int rcv_bn_finalize_apply(int32_t N, int32_t C, int64_t HW, const double* stats, const float* gamma,
-                                     const float* beta, float* running_mean, float* running_var, float momentum,
-                                     float eps, const float* z, int relu, const float* residual,
-                                     int32_t res_channels, float* y,
-                                     float* scale, float* shift, float* save_mean, float* save_invstd,
-                                     int64_t* num_batches_tracked, void* stream) {
-  RCV_REQUIRE(N > 0 && C > 0 && HW > 0 && stats && z && y && scale && shift, RCV_ERR_BAD_ARG,
+// the statistics in `stats` were summed over `count_` elements per channel: N*HW on one rank, more when the sums were
+// added up over the ranks of a global batch (TrainStep(global_batch=True))
+extern "C" int rcv_bn_finalize_apply_count(int32_t N, int32_t C, int64_t HW, int64_t count_, const double* stats,
+                                           const float* gamma, const float* beta, float* running_mean,
+                                           float* running_var, float momentum, float eps, const float* z, int relu,
+                                           const float* residual, int32_t res_channels, float* y, float* scale,
+                                           float* shift, float* save_mean, float* save_invstd,
+                                           int64_t* num_batches_tracked, void* stream) {
+  RCV_REQUIRE(N > 0 && C > 0 && HW > 0 && count_ > 0 && stats && z && y && scale && shift, RCV_ERR_BAD_ARG,
               "bn_finalize_apply: bad arg");
   RCV_REQUIRE(C <= 4096, RCV_ERR_UNSUPPORTED, "bn_finalize_apply: C=%d > 4096", C);
   const int64_t total = (int64_t)N * C * HW;
-  const double count = (double)N * (double)HW;
+  const double count = (double)count_;
   const size_t smem = (size_t)2 * C * sizeof(float);
   RCV_REQUIRE(res_channels >= 0 && res_channels <= C, RCV_ERR_BAD_ARG, "bn_finalize_apply: res_channels %d outside [0, %d]",
               res_channels, C);
@@ -604,6 +606,17 @@ extern "C" int rcv_bn_finalize_apply(int32_t N, int32_t C, int64_t HW, const dou
                scale, shift, save_mean, save_invstd, reinterpret_cast<long long*>(num_batches_tracked));
   RCV_CHECK_LAUNCH("bn_finalize_apply");
   return RCV_OK;
+}
+
+extern "C" int rcv_bn_finalize_apply(int32_t N, int32_t C, int64_t HW, const double* stats, const float* gamma,
+                                     const float* beta, float* running_mean, float* running_var, float momentum,
+                                     float eps, const float* z, int relu, const float* residual,
+                                     int32_t res_channels, float* y,
+                                     float* scale, float* shift, float* save_mean, float* save_invstd,
+                                     int64_t* num_batches_tracked, void* stream) {
+  return rcv_bn_finalize_apply_count(N, C, HW, (int64_t)N * HW, stats, gamma, beta, running_mean, running_var,
+                                     momentum, eps, z, relu, residual, res_channels, y, scale, shift, save_mean,
+                                     save_invstd, num_batches_tracked, stream);
 }
 
 extern "C" int rcv_bn_bwd_reduce(int32_t N, int32_t C, int64_t HW, int order, const float* dy,

@@ -20,6 +20,8 @@
 
 #include <stdlib.h>
 
+#include <type_traits>
+
 namespace {
 
 constexpr int NT = 256;
@@ -123,6 +125,89 @@ __global__ void __launch_bounds__(NT) peer_allreduce_kernel(PeerArgs pa, int ran
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Small-vector exchange (TrainStep(global_batch=True)): buf[off, off+count) <- scale * sum over ranks, for the few
+// hundred fp64 / int64 values of a BatchNorm layer's statistics or backward sums, a loss normaliser or a correct count.
+// ONE CTA: every rank loads all N copies and writes only its own buffer, in place.  The order of the steps is what
+// makes the in-place write safe:
+//   1. ready barrier: "my values are final" (the kernel boundary before it made them visible);
+//   2. load all N copies, add them in rank order (the same bits on every rank), keep the sums in shared memory;
+//   3. done barrier: "I have read yours";
+//   4. store the scaled sums into the local buffer.
+// No peer can read a value after it was overwritten: a rank writes only after every peer has posted that its loads
+// are done.  A rank's next write into the same buffer (the next step's memset, the next layer's statistics) follows
+// its own launch in stream order, hence also every peer's loads.  Same flag words, launch counts and time-out as
+// peer_allreduce_kernel: a slot must be used by one stream of each rank at a time.
+constexpr int SMALL_MAX = 4096;  // elements per launch (32 KB of shared memory)
+
+struct SmallArgs {
+  void* buf[PEER_MAX];
+  uint32_t* flags[PEER_MAX];
+};
+
+__device__ __forceinline__ double ld_peer_elem(const double* p) {
+  double v;
+  asm volatile("ld.relaxed.sys.global.f64 %0, [%1];" : "=d"(v) : "l"(p) : "memory");
+  return v;
+}
+__device__ __forceinline__ long long ld_peer_elem(const long long* p) {
+  long long v;
+  asm volatile("ld.relaxed.sys.global.s64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+  return v;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(NT) peer_small_allreduce_kernel(SmallArgs pa, int world, int rank, int slot,
+                                                                  int64_t off, int count, double scale,
+                                                                  uint64_t timeout_ns, int32_t* status) {
+  rcv_pdl_enter();
+  __shared__ T s_sum[SMALL_MAX];
+  __shared__ uint32_t s_epoch;
+  __shared__ int s_fail;
+  uint32_t* mine = pa.flags[rank] + slot * SLOT_WORDS;
+  if (threadIdx.x == 0) {
+    s_epoch = *reinterpret_cast<volatile uint32_t*>(mine + 32) + 1;
+    s_fail = 0;
+  }
+  __syncthreads();
+  const uint32_t epoch = s_epoch;
+  // 1. ready barrier
+  __threadfence_system();
+  if (threadIdx.x < world) st_release_sys(pa.flags[threadIdx.x] + slot * SLOT_WORDS + rank, epoch);
+  if (threadIdx.x < world && !wait_flag(mine + threadIdx.x, epoch, timeout_ns)) s_fail = 1;
+  __syncthreads();
+  const bool ok = !s_fail;
+  // 2. every rank's copy, summed in rank order
+  if (ok) {
+    for (int i = threadIdx.x; i < count; i += NT) {
+      T s = ld_peer_elem(reinterpret_cast<const T*>(pa.buf[0]) + off + i);
+      for (int q = 1; q < world; ++q) s += ld_peer_elem(reinterpret_cast<const T*>(pa.buf[q]) + off + i);
+      s_sum[i] = s;
+    }
+  }
+  // 3. done barrier: the loads above are complete before any peer hears of it
+  __threadfence_system();
+  __syncthreads();
+  if (ok) {
+    if (threadIdx.x < world) st_release_sys(pa.flags[threadIdx.x] + slot * SLOT_WORDS + 16 + rank, epoch);
+    if (threadIdx.x < world && !wait_flag(mine + 16 + threadIdx.x, epoch, timeout_ns)) s_fail = 1;
+  }
+  __syncthreads();
+  if (s_fail) {  // a peer never arrived: leave the buffer alone and report
+    if (threadIdx.x == 0) atomicExch(status, 1);
+  } else {
+    // 4. the local result, in place
+    T* dst = reinterpret_cast<T*>(pa.buf[rank]) + off;
+    for (int i = threadIdx.x; i < count; i += NT) {
+      if constexpr (std::is_same<T, double>::value)
+        dst[i] = s_sum[i] * scale;
+      else
+        dst[i] = s_sum[i];  // integer counts: exact sums, no scale
+    }
+  }
+  if (threadIdx.x == 0) *reinterpret_cast<volatile uint32_t*>(mine + 32) = epoch;
+}
+
 uint64_t timeout_ns() {
   static uint64_t ns = [] {
     const char* e = getenv("RCV_PEER_TIMEOUT_S");
@@ -215,4 +300,46 @@ extern "C" int rcv_peer_allreduce(int32_t world, int32_t rank, int32_t slot, flo
 #undef RCV_PEER_CASE
   RCV_CHECK_LAUNCH("peer_allreduce");
   return RCV_OK;
+}
+
+namespace {
+
+template <typename T>
+int peer_small_allreduce(const char* name, int32_t world, int32_t rank, int32_t slot, T* const* bufs,
+                         uint32_t* const* flags, int64_t offset, int64_t count, double scale, int32_t* status,
+                         void* stream) {
+  RCV_REQUIRE(world >= 1 && world <= PEER_MAX && rank >= 0 && rank < world && bufs && flags && status,
+              RCV_ERR_BAD_ARG, "%s: bad arg (world %d, rank %d)", name, world, rank);
+  RCV_REQUIRE(slot >= 0 && slot < PEER_SLOTS, RCV_ERR_BAD_ARG, "%s: slot %d of %d", name, slot, PEER_SLOTS);
+  RCV_REQUIRE(offset >= 0 && count > 0 && count <= SMALL_MAX, RCV_ERR_BAD_ARG,
+              "%s: offset %lld / count %lld (1..%d elements)", name, (long long)offset, (long long)count, SMALL_MAX);
+  SmallArgs pa;
+  memset(&pa, 0, sizeof(pa));
+  for (int q = 0; q < world; ++q) {
+    RCV_REQUIRE(bufs[q] && flags[q] && ((uintptr_t)bufs[q] % sizeof(T) == 0), RCV_ERR_BAD_ARG,
+                "%s: buffer / flags of rank %d", name, q);
+    pa.buf[q] = bufs[q];
+    pa.flags[q] = flags[q];
+  }
+  rcv_launch(peer_small_allreduce_kernel<T>, dim3(1), dim3(NT), 0, (cudaStream_t)stream, pa, (int)world, (int)rank,
+             (int)slot, offset, (int)count, scale, timeout_ns(), status);
+  RCV_CHECK_LAUNCH(name);
+  return RCV_OK;
+}
+
+}  // namespace
+
+extern "C" int rcv_peer_allreduce_f64(int32_t world, int32_t rank, int32_t slot, double* const* bufs,
+                                      uint32_t* const* flags, int64_t offset, int64_t count, double scale,
+                                      int32_t* status, void* stream) {
+  return peer_small_allreduce<double>("peer_allreduce_f64", world, rank, slot, bufs, flags, offset, count, scale,
+                                      status, stream);
+}
+
+extern "C" int rcv_peer_allreduce_i64(int32_t world, int32_t rank, int32_t slot, int64_t* const* bufs,
+                                      uint32_t* const* flags, int64_t offset, int64_t count, int32_t* status,
+                                      void* stream) {
+  return peer_small_allreduce<long long>("peer_allreduce_i64", world, rank, slot,
+                                         reinterpret_cast<long long* const*>(bufs), flags, offset, count, 1.0, status,
+                                         stream);
 }

@@ -79,7 +79,7 @@ def allreduce_buckets(flat, buckets: Sequence[Tuple[int, int, int]], group=None)
 
 def self_check(model_ctor, class_weights, batch: int, cin: int, h: int, w: int, steps: int = 3, group=None,
                lr: float = 1e-3, l1_decay: float = 1e-6, seed: int = 777, use_graph: bool = True,
-               force_comm_path: bool = True, tol: float = 5e-4, reduce=None) -> dict:
+               force_comm_path: bool = True, tol: float = 5e-4, reduce=None, global_batch: bool = False) -> dict:
     """Numerical check of the data-parallel product path on THIS job's ranks (bench.py emits it as `dp_check`).
 
     Every rank trains `steps` steps of TrainStep (bucketed all-reduce + optimiser on the comm stream, captured in a
@@ -93,6 +93,8 @@ def self_check(model_ctor, class_weights, batch: int, cin: int, h: int, w: int, 
     by up to ~1e-4 here (floating-point atomics in the weight-gradient kernels, passed on by Adam's normalisation:
     the control in tests/test_gpu_train.py::test_comm_path_schedule_matches_plain_step); a missing or mis-scaled
     all-reduce, or an optimiser pass racing a gradient, moves weights by the order of lr = 1e-3 per step.
+    global_batch: check TrainStep(global_batch=True) instead; the serial reference is then one process stepping on
+    the N shards concatenated into one batch (BatchNorm statistics and loss over all of it).
 
     -> {"ok", "world", "steps", "max_weight_err", "max_loss_err", "weights_identical_across_ranks"}"""
     import copy
@@ -114,7 +116,7 @@ def self_check(model_ctor, class_weights, batch: int, cin: int, h: int, w: int, 
     emu = copy.deepcopy(model)
     eps = 1e-3
     ts = TrainStep(model, class_weights, lr=lr, l1_decay=l1_decay, eps=eps, use_graph=use_graph,
-                   process_group=group, force_comm_path=force_comm_path, reduce=reduce)
+                   process_group=group, force_comm_path=force_comm_path, reduce=reduce, global_batch=global_batch)
     crit = CrossEntropyLoss2d(torch.tensor(class_weights)).to(dev)
     opt = torch.optim.Adam(emu.parameters(), lr=lr, eps=eps)
     gen = torch.Generator().manual_seed(seed)
@@ -127,7 +129,11 @@ def self_check(model_ctor, class_weights, batch: int, cin: int, h: int, w: int, 
         dp_loss = float(ts.loss_sums[0] / ts.loss_sums[1])
         emu.train()
         opt.zero_grad()
-        for r in range(world):
+        if global_batch:
+            loss_g = crit(emu(xs.flatten(0, 1)), ys.flatten(0, 1))
+            max_loss = max(max_loss, abs(float(loss_g.detach()) - dp_loss) / max(1.0, abs(dp_loss)))
+            loss_g.backward()
+        for r in range(0 if global_batch else world):
             loss_r = crit(emu(xs[r].contiguous()), ys[r].contiguous())
             if r == rank:
                 max_loss = max(max_loss, abs(float(loss_r.detach()) - dp_loss) / max(1.0, abs(dp_loss)))

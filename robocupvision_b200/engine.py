@@ -273,12 +273,16 @@ class Plan:
         return len(self.nodes) - 1
 
     def forward(self, x: torch.Tensor, training: bool, save: bool, stats_arena: Optional[torch.Tensor] = None,
-                stop_before: Optional[int] = None):
+                stop_before: Optional[int] = None, batch_reduce=None):
         """-> (outputs, saved).  training selects batch statistics for BatchNorm nodes whose
         module is in training mode; save keeps what backward needs.  stats_arena: caller-zeroed float64[n_stats]
         for the batch statistics (TrainStep zeroes all of a step's accumulators with one memset).
         stop_before: run nodes [0, stop_before) only (TrainStep's fused head); outputs that were not produced are
-        None, and backward() then starts from the `seed` gradients it is given."""
+        None, and backward() then starts from the `seed` gradients it is given.
+        batch_reduce: BatchNorm over a batch split across ranks (TrainStep(global_batch=True)) -- an object with
+        `world` and `sum(buf)` / `mean(buf)`, which replace a float64 slice by its sum / mean over the ranks in place
+        on the current stream.  Every train-mode BatchNorm's statistics are summed between its conv and its finalize,
+        which then divides by the global count (this rank's N*H*W times world; every rank holds as many samples)."""
         x = ops._chk(x, name="input")
         if x.dim() != 4:
             raise ValueError(f"expected NCHW input, got shape {tuple(x.shape)}")
@@ -329,6 +333,9 @@ class Plan:
                 z = ops.conv_fwd(g, src, w, b, epilogue=EPI_RELU if nd.order == EPI_RELU_AFFINE else EPI_NONE,
                                  stats=stats, math=self.math, wpacked=wp, in_affine=ina, workspace=ws)
                 count = z.numel() // g.cout
+                if batch_reduce is not None:
+                    batch_reduce.sum(stats)
+                    count *= batch_reduce.world
                 if bn.momentum is None:
                     momentum = 1.0 / float(int(bn.num_batches_tracked) + 1)
                 else:
@@ -345,7 +352,8 @@ class Plan:
                     y, scale, shift, mean, invstd = ops.bn_finalize_apply(
                         z, stats, bn.weight.detach(), bn.bias.detach(),
                         bn.running_mean if track else None, bn.running_var if track else None, momentum, bn.eps,
-                        relu=(nd.order == EPI_AFFINE_RELU), residual=skip, num_batches_tracked=nbt)
+                        relu=(nd.order == EPI_AFFINE_RELU), residual=skip, num_batches_tracked=nbt,
+                        **({} if batch_reduce is None else {"count": count}))
                 saved[t] = (z, scale, shift, mean, invstd)
             else:
                 scale, shift = nd.folded(self.epoch)
@@ -362,12 +370,17 @@ class Plan:
     # ------------------------------------------------------------------ backward
     def backward(self, saved_all, gouts: Sequence[Optional[torch.Tensor]], x_needs_grad: bool,
                  grad_views: Optional[Dict[int, torch.Tensor]] = None, node_done=None,
-                 sums_arena: Optional[torch.Tensor] = None, seed: Optional[Dict[int, torch.Tensor]] = None):
+                 sums_arena: Optional[torch.Tensor] = None, seed: Optional[Dict[int, torch.Tensor]] = None,
+                 batch_reduce=None):
         """-> (dx or None, {id(param): grad}).  grad_views, if given, maps id(param) to zero-filled
         tensors that receive the gradients (the train step's flat arena).  node_done(t) is called
         once node t's parameter gradients are final (nodes are visited last to first).  sums_arena: caller-zeroed
         float64[n_stats] for the BatchNorm-backward sums.  seed: {activation index: gradient} for a forward that
-        stopped early (forward(stop_before=...)): the nodes that did not run are skipped, node_done still sees them."""
+        stopped early (forward(stop_before=...)): the nodes that did not run are skipped, node_done still sees them.
+        batch_reduce: as for forward(); every BatchNorm backward then runs as its two passes with the channel sums
+        averaged over the ranks between them.  The apply pass divides by this rank's N*H*W, so the averaged sums give
+        the global means; the dgamma / dbeta it adds are the averages, which the sum all-reduce of the gradients
+        turns back into the global sums."""
         acts, saved, lazy = saved_all
         lazy_done: Dict[int, torch.Tensor] = {}  # BatchNorm outputs materialised for a weight gradient, per activation
         dev = acts[0].device
@@ -404,7 +417,7 @@ class Plan:
         for t in range(len(self.nodes) - 1, -1, -1):
             if t + 1 < len(acts):  # (a node the forward pass stopped before has no activation and no gradient)
                 self._backward_node(t, acts, saved, grads, grad_views, sums_arena, x_needs_grad, add_to, side, keep,
-                                    lazy, lazy_done)
+                                    lazy, lazy_done, batch_reduce)
             if node_done is not None:
                 node_done(t)
         if side is not None:
@@ -413,7 +426,7 @@ class Plan:
         return grads[0], grad_views
 
     def _backward_node(self, t, acts, saved, grads, grad_views, sums_arena, x_needs_grad, add_to, side=None,
-                       keep=None, lazy=None, lazy_done=None):
+                       keep=None, lazy=None, lazy_done=None, batch_reduce=None):
         nd = self.nodes[t]
         g = grads[t + 1]
         grads[t + 1] = None
@@ -445,9 +458,16 @@ class Plan:
                     "backward through an eval-mode BatchNorm block is not on the hot path "
                     "(call model.train() before the forward pass you differentiate)")
             z, scale, shift, mean, invstd = saved[t]
-            dconv, _, _, _ = ops.bn_bwd(nd.order, g, z, scale, shift, mean, invstd,
-                                        dgamma=grad_views[id(bn.weight)], dbeta=grad_views[id(bn.bias)],
-                                        dbias=grad_views[id(conv.bias)] if has_bias else None, sums=sums)
+            dbias = grad_views[id(conv.bias)] if has_bias else None
+            if batch_reduce is None:
+                dconv, _, _, _ = ops.bn_bwd(nd.order, g, z, scale, shift, mean, invstd,
+                                            dgamma=grad_views[id(bn.weight)], dbeta=grad_views[id(bn.bias)],
+                                            dbias=dbias, sums=sums)
+            else:
+                ops.bn_bwd_reduce(nd.order, g, z, scale, shift, mean, invstd, sums)
+                batch_reduce.mean(sums)
+                dconv = ops.bn_bwd_apply(nd.order, g, z, scale, shift, mean, invstd, sums,
+                                         dgamma=grad_views[id(bn.weight)], dbeta=grad_views[id(bn.bias)], dbias=dbias)
             wg_bias = None
         else:
             dconv = ops.relu_bwd(g, saved[t][0]) if nd.order == EPI_RELU else g

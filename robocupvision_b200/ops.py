@@ -19,7 +19,7 @@ from ._lib import (DET_CE_FWD, DET_CE_WEIGHT_SUM, DET_DICE_FWD, DET_L1_SUM, ENGI
 
 __all__ = [
     "ConvGeom", "conv_fwd", "conv_dgrad", "conv_wgrad", "conv_pack", "conv_packed_bytes", "conv_workspace_bytes", "new_workspace", "conv_takes_partial_residual", "conv_uses_tensor_cores", "conv_engine", "conv_normalises_on_load", "PackTable", "bn_finalize_apply", "PACK_FWD", "PACK_DGRAD", "bn_finalize", "bn_fold", "bn_apply",
-    "bn_bwd", "relu_bwd", "channel_sum", "maxpool2x2_fwd", "maxpool2x2_bwd", "maxunpool2x2", "maxunpool2x2_bwd", "upsample_bilinear2x", "upsample_bilinear2x_bwd", "ce_fwd", "ce_bwd",
+    "bn_bwd", "bn_bwd_reduce", "bn_bwd_apply", "relu_bwd", "channel_sum", "maxpool2x2_fwd", "maxpool2x2_bwd", "maxunpool2x2", "maxunpool2x2_bwd", "upsample_bilinear2x", "upsample_bilinear2x_bwd", "ce_fwd", "ce_bwd",
     "confusion", "metric_tail", "mask_label_lut", "mask_label_", "label_to_pred", "lp_assemble", "augment", "color_jitter_params", "dice_fwd", "dice_bwd", "dice_loss", "head_dice_fwd", "head_dice_train", "adam_l1_step", "sgd_step", "det_scratch_bytes", "det_scratch", "zero_", "zeros", "counter_add", "launch_count", "reset_launch_count",
     "EPI_NONE", "EPI_RELU", "EPI_RELU_AFFINE", "EPI_AFFINE_RELU", "EPI_AFFINE",
     "DET_CE_FWD", "DET_CE_WEIGHT_SUM", "DET_DICE_FWD", "DET_L1_SUM",
@@ -211,9 +211,10 @@ def _res_channels(residual, c):
 
 
 def bn_finalize_apply(z, stats, gamma, beta, running_mean, running_var, momentum, eps, relu, residual=None,
-                      num_batches_tracked=None):
+                      num_batches_tracked=None, count=None):
     """Train-mode BatchNorm forward in one launch -> (y, scale, shift, mean, invstd).  A residual with fewer channels
-    than z is added to the first channels only."""
+    than z is added to the first channels only.  count: elements per channel the statistics were summed over
+    (rcv_bn_finalize_apply_count; statistics summed over the ranks of a global batch), default N*HW of z."""
     z = _chk(z, name="z")
     n, c = z.shape[0], z.shape[1]
     hw = z.numel() // (n * c)
@@ -221,7 +222,9 @@ def bn_finalize_apply(z, stats, gamma, beta, running_mean, running_var, momentum
     y = torch.empty_like(z)
     if residual is not None:
         residual = _chk(residual, name="residual")
-    _call("rcv_bn_finalize_apply", 1, n, c, hw, _ptr(stats), _ptr(gamma), _ptr(beta), _ptr(running_mean),
+    head = ("rcv_bn_finalize_apply", 1, n, c, hw) if count is None else (
+        "rcv_bn_finalize_apply_count", 1, n, c, hw, int(count))
+    _call(*head, _ptr(stats), _ptr(gamma), _ptr(beta), _ptr(running_mean),
           _ptr(running_var), float(momentum), float(eps), _ptr(z), 1 if relu else 0, _ptr(residual),
           _res_channels(residual, c), _ptr(y),
           _ptr(buf[0]), _ptr(buf[1]), _ptr(buf[2]), _ptr(buf[3]), _ptr(num_batches_tracked), _stream())
@@ -381,6 +384,35 @@ def bn_bwd(order: int, dy, z, scale, shift, mean, invstd, dgamma=None, dbeta=Non
     _call("rcv_bn_bwd", 1 if fused else 2, n, c, hw, order, _ptr(dy), _ptr(z), _ptr(scale), _ptr(shift), _ptr(mean),
           _ptr(invstd), _ptr(sums), _ptr(dconv), _ptr(dgamma), _ptr(dbeta), _ptr(dbias), st)
     return dconv, dgamma, dbeta, dbias
+
+
+def bn_bwd_reduce(order: int, dy, z, scale, shift, mean, invstd, sums) -> None:
+    """Pass 1 of the BatchNorm backward alone: sums[c] += sum(g), sums[C+c] += sum(g*xhat) (float64[2C], zeroed by the
+    caller).  With bn_bwd_apply it is bn_bwd in two launches, with the sums in memory between them (a global batch
+    averages them over the ranks there)."""
+    dy = _chk(dy, name="dy")
+    z = _chk(z, name="z")
+    n, c = z.shape[0], z.shape[1]
+    hw = z.numel() // (n * c)
+    if sums.dtype != torch.float64 or sums.numel() != 2 * c:
+        raise ValueError("bn_bwd_reduce: sums must be float64[2*C]")
+    _call("rcv_bn_bwd_reduce", 1, n, c, hw, order, _ptr(dy), _ptr(z), _ptr(scale), _ptr(shift), _ptr(mean),
+          _ptr(invstd), _ptr(sums), _stream())
+
+
+def bn_bwd_apply(order: int, dy, z, scale, shift, mean, invstd, sums, dgamma=None, dbeta=None, dbias=None):
+    """Pass 2 of the BatchNorm backward: -> dconv from the channel sums of bn_bwd_reduce (means = sums / (N*HW) of
+    this z); dgamma += sums[C:], dbeta += sums[:C], dbias += sum(dconv) where given."""
+    dy = _chk(dy, name="dy")
+    z = _chk(z, name="z")
+    n, c = z.shape[0], z.shape[1]
+    hw = z.numel() // (n * c)
+    if sums.dtype != torch.float64 or sums.numel() != 2 * c:
+        raise ValueError("bn_bwd_apply: sums must be float64[2*C]")
+    dconv = torch.empty_like(z)
+    _call("rcv_bn_bwd_apply", 1, n, c, hw, order, _ptr(dy), _ptr(z), _ptr(scale), _ptr(shift), _ptr(mean),
+          _ptr(invstd), _ptr(sums), _ptr(dconv), _ptr(dgamma), _ptr(dbeta), _ptr(dbias), _stream())
+    return dconv
 
 
 def relu_bwd(dy, y):

@@ -88,7 +88,8 @@ class TrainStep:
                  weight_decay: float = 0.0, lr_mults: Optional[Sequence] = None,
                  process_group=None, use_graph: bool = True, overlap_comm: bool = True, n_buckets: int = 3,
                  force_comm_path: bool = False, reduce: Optional[str] = None,
-                 fused_head: bool = _FUSED_HEAD, loss: str = "ce", dice_eps: float = 1e-7):
+                 fused_head: bool = _FUSED_HEAD, loss: str = "ce", dice_eps: float = 1e-7,
+                 global_batch: bool = False):
         """masks: pruneModelNew-style list of bool tensors for the >1-D parameters, in parameter
         order (train.py:59-65); with masks the L1 term is dropped (train.py:53).
         optimizer: "adam" (train.py:357-363; torch defaults, no weight decay) or "sgd" (trainer.py:182-184:
@@ -113,7 +114,15 @@ class TrainStep:
         sums are rank-local and the gradients averaged: each rank's loss is the Dice loss of its own shard, the
         semantics DistributedDataParallel gives the reference's loop.
         The optimiser passes of the buckets run on the side stream with one rank too (overlap_comm): they overlap the
-        encoder's backward (+0.5 % on the single-GPU step)."""
+        encoder's backward (+0.5 % on the single-GPU step).
+        global_batch: the N ranks, each holding B/N samples (the same shape on every rank), train ONE batch of B: what
+        one process computes on all B samples, up to floating-point rounding -- BatchNorm batch statistics (summed
+        over the ranks; the running variance's unbiased factor from the global count), BatchNorm backward, the CE
+        normaliser sum(w[y]), the Dice sums, and the reported loss and correct count.  The small fp64 / int64 vectors
+        are exchanged on the main stream in the middle of the step (rcv_peer_allreduce_f64 / _i64 over peer memory,
+        dist.all_reduce under reduce="nccl"), and the gradients are summed over the ranks instead of averaged.
+        Without it every rank's BatchNorm and loss see its own shard only (DistributedDataParallel's semantics).
+        With one rank it changes nothing unless force_comm_path runs the exchanges (at world 1)."""
         if loss not in ("ce", "dice"):
             raise ValueError(f"TrainStep: loss must be 'ce' or 'dice', got {loss!r}")
         if optimizer not in ("adam", "sgd"):
@@ -121,12 +130,34 @@ class TrainStep:
         if optimizer == "adam" and (weight_decay != 0.0 or momentum != 0.0):
             raise ValueError("TrainStep: optimizer='adam' is torch.optim.Adam with its defaults (train.py:357-363): "
                              "weight_decay and momentum must be 0 (they belong to optimizer='sgd')")
+        asked = reduce or os.environ.get("RCV_B200_DP_REDUCE", "")
+        if asked not in ("", "peer", "nccl"):
+            raise ValueError(f"TrainStep: reduce must be 'peer' or 'nccl', got {asked!r}")
         self.model = model
         self.plan: Plan = model._get_plan()
         dev = next(model.parameters()).device
         if dev.type != "cuda":
             raise RuntimeError("TrainStep needs the model on a CUDA device (no CPU path)")
         self.dev = dev
+        self.loss = loss
+        self.dice_eps = float(dice_eps)
+        if loss == "dice":
+            if len(self.plan.outputs) != 1 or self.plan.nodes[self.plan.outputs[0] - 1].kind != "conv":
+                raise ValueError("TrainStep(loss='dice'): the plan must end in one classifier conv")
+            ncls = self.plan.nodes[self.plan.outputs[0] - 1].geom.cout
+            w = torch.ones(ncls) if class_weights is None else torch.as_tensor(class_weights, dtype=torch.float32)
+            if w.numel() != ncls:
+                raise ValueError(f"TrainStep(loss='dice'): {w.numel()} class weights for {ncls} classes")
+            class_weights = w / w.sum().item() * w.shape[0]  # DiceLoss.__init__
+        self.class_w = None if class_weights is None else torch.as_tensor(
+            class_weights, dtype=torch.float32).to(dev)
+        # every small accumulator of a step in ONE buffer (one memset per step):
+        # [l1 sum | CE loss sums (2) | correct pixels (int64 view) | BN batch statistics | BN backward sums]
+        # loss="dice" appends [Dice sums (2C) | the unused loss sums of the correct-count pass of the unfused head (2)]
+        # and keeps [dice loss, 1.0] where the CE loss sums are
+        ns = self.plan.n_stats
+        ndice = 2 * self.class_w.numel() + 2 if loss == "dice" else 0
+        n_acc = 4 + 2 * ns + ndice
         self.arena, self.table = flatten_parameters(model)
         n = self.arena.numel()
         self.pg = process_group
@@ -134,16 +165,14 @@ class TrainStep:
         if process_group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()):
             self.world = torch.distributed.get_world_size(process_group)
         force_comm_path = force_comm_path or os.environ.get("RCV_B200_FORCE_COMM_PATH", "") == "1"
-        asked = reduce or os.environ.get("RCV_B200_DP_REDUCE", "")
-        if asked not in ("", "peer", "nccl"):
-            raise ValueError(f"TrainStep: reduce must be 'peer' or 'nccl', got {asked!r}")
         self.reduce = asked or "peer"
         self.peer = None
         self.grads = None
         if self.reduce == "peer" and (self.world > 1 or force_comm_path):
             from .peer import PeerExchange, PeerUnavailable
             try:
-                self.peer = PeerExchange(n, dev, group=process_group)
+                # under global_batch the accumulators live in the peer-mapped block too, so the peers can read them
+                self.peer = PeerExchange(n, dev, group=process_group, ndoubles=n_acc if global_batch else 0)
                 self.grads = self.peer.grads
             except PeerUnavailable as e:  # raised on every rank or on none
                 if asked == "peer":
@@ -154,6 +183,10 @@ class TrainStep:
                 self.reduce = "nccl"
         if self.world == 1 and self.peer is None:
             self.reduce = "none"
+        # a global batch needs an exchange: none with one rank unless force_comm_path put the peer path in place
+        self.global_batch = bool(global_batch) and self.reduce != "none"
+        self._batch_reduce = _RankReduce(self) if self.global_batch else None
+        self._shard_shape = None
         if self.grads is None:
             self.grads = _zeros(n, torch.float32, dev)
         if self.world > 1 and "RCV_PDL" not in os.environ:
@@ -177,18 +210,6 @@ class TrainStep:
                 if p.dim() > 1:
                     self.mask[o:o + k] = masks[i].reshape(-1).to(dev).to(torch.uint8)
                     i += 1
-        self.loss = loss
-        self.dice_eps = float(dice_eps)
-        if loss == "dice":
-            if len(self.plan.outputs) != 1 or self.plan.nodes[self.plan.outputs[0] - 1].kind != "conv":
-                raise ValueError("TrainStep(loss='dice'): the plan must end in one classifier conv")
-            ncls = self.plan.nodes[self.plan.outputs[0] - 1].geom.cout
-            w = torch.ones(ncls) if class_weights is None else torch.as_tensor(class_weights, dtype=torch.float32)
-            if w.numel() != ncls:
-                raise ValueError(f"TrainStep(loss='dice'): {w.numel()} class weights for {ncls} classes")
-            class_weights = w / w.sum().item() * w.shape[0]  # DiceLoss.__init__
-        self.class_w = None if class_weights is None else torch.as_tensor(
-            class_weights, dtype=torch.float32).to(dev)
         # lr groups: contiguous arena ranges (padding included) with a multiplier
         mult = torch.ones(len(self.table))
         if lr_mults:
@@ -218,13 +239,8 @@ class TrainStep:
         self._lr_host = torch.tensor([lr * r[2] for r in self.ranges], dtype=torch.float32).pin_memory()
         self.lr_dev = self._lr_host.to(dev)
         self.step_dev = _zeros(1, torch.int32, dev)
-        # every small accumulator of a step in ONE buffer (one memset per step):
-        # [l1 sum | CE loss sums (2) | correct pixels (int64 view) | BN batch statistics | BN backward sums]
-        # loss="dice" appends [Dice sums (2C) | the unused loss sums of the correct-count pass of the unfused head (2)]
-        # and keeps [dice loss, 1.0] where the CE loss sums are
-        ns = self.plan.n_stats
-        ndice = 2 * self.class_w.numel() + 2 if loss == "dice" else 0
-        self._accum = _zeros(4 + 2 * ns + ndice, torch.float64, dev)
+        self._accum = (self.peer.accum if self.global_batch and self.peer is not None
+                       else _zeros(n_acc, torch.float64, dev))
         self._acc_l1, self._acc_ce = self._accum[0:1], self._accum[1:3]
         self._acc_corr = self._accum[3:4].view(torch.int64)
         self._acc_stats, self._acc_sums = self._accum[4:4 + ns], self._accum[4 + ns:4 + 2 * ns]
@@ -236,6 +252,11 @@ class TrainStep:
         # (first plan node, arena start, arena end), in the order backward completes them (arena tail first)
         self.buckets = dp.plan_buckets([[self.offsets[id(p)] for p in nd.params()] for nd in self.plan.nodes],
                                        [(o, k) for _, o, k in self.table], n, n_buckets) if self.comm_path else []
+        if self.global_batch and self.peer is not None:
+            from .peer import SMALL_SLOT
+            if len(self.buckets) > SMALL_SLOT:
+                raise ValueError(f"TrainStep(global_batch=True): at most {SMALL_SLOT} gradient buckets, "
+                                 f"got {len(self.buckets)}")
         # the classifier head in one pass (ops.head_ce_train; two for Dice) where the plan ends in a bare 1x1 conv the
         # kernel covers
         self._head = self.plan.fusable_head() if fused_head else -1
@@ -283,9 +304,24 @@ class TrainStep:
         elif self.world > 1 or self.pg is not None:
             torch.distributed.all_reduce(self.grads[a:b], group=self.pg)
 
+    def _reduce_f64(self, t: torch.Tensor, scale: float = 1.0):
+        """t (a float64 slice of the accumulator buffer) <- scale * sum over ranks, on the current stream."""
+        if self.peer is not None:
+            self.peer.allreduce_f64(t, scale)
+        else:
+            dist = torch.distributed
+            dist.all_reduce(t, op=dist.ReduceOp.SUM if scale == 1.0 else dist.ReduceOp.AVG, group=self.pg)
+
+    def _reduce_i64(self, t: torch.Tensor):
+        """t (an int64 view of the accumulator buffer) <- sum over ranks, on the current stream."""
+        if self.peer is not None:
+            self.peer.allreduce_i64(t)
+        else:
+            torch.distributed.all_reduce(t, group=self.pg)
+
     def _optim_range(self, a: int, b: int, l1):
         """Optimiser pass over arena[a:b), split at the lr-group boundaries."""
-        gscale = 1.0 / self.world
+        gscale = 1.0 if self.global_batch else 1.0 / self.world  # a global batch's gradient is the sum over ranks
         for i, (ra, rb, _) in enumerate(self.ranges):
             lo, hi = max(a, ra), min(b, rb)
             if lo >= hi:
@@ -314,12 +350,15 @@ class TrainStep:
         ops.counter_add(self.step_dev, 1)
         head = self._head
         seed = None
+        gb = self._batch_reduce
         if head >= 0 and self.loss == "ce":
             # the normaliser of the weighted mean loss depends on the labels only: produced here, so that the head
             # needs ONE pass (classifier conv + loss + argmax + their backward, ops.head_ce_train)
             ops.ce_weight_sum(y, self.class_w, self._acc_ce[1:2], self.plan.nodes[head].geom.cout)
+            if gb is not None:
+                self._reduce_f64(self._acc_ce[1:2])  # the head divides by the global normaliser
         outs, saved = self.plan.forward(x, training=True, save=True, stats_arena=self._acc_stats,
-                                        stop_before=head if head >= 0 else None)
+                                        stop_before=head if head >= 0 else None, batch_reduce=gb)
         if head >= 0 and saved[2].get(self.plan.nodes[head].src) is not None:
             raise RuntimeError("TrainStep: the classifier reads a BatchNorm that was deferred to its consumer")
         sums, corr = self._acc_ce, self._acc_corr
@@ -336,6 +375,8 @@ class TrainStep:
             logits = outs[0]
             sums, _, _, corr = ops.ce_fwd(logits, y, self.class_w, want_correct=True, sums=self._acc_ce,
                                           corr=self._acc_corr)
+            if gb is not None:
+                self._reduce_f64(self._acc_ce)  # ce_bwd divides by the global normaliser
             gouts = [ops.ce_bwd(logits, y, self.class_w, sums)]
         if self.comm_path:
             cur = torch.cuda.current_stream()
@@ -353,14 +394,20 @@ class TrainStep:
                         self._allreduce(a, b, slot=k)
                         self._optim_range(a, b, l1)
             self.plan.backward(saved, gouts, False, self.grad_views, node_done=flush, sums_arena=self._acc_sums,
-                               seed=seed)
+                               seed=seed, batch_reduce=gb)
             flush(-1)
             cur.wait_stream(self.comm_stream)
         else:
-            self.plan.backward(saved, gouts, False, self.grad_views, sums_arena=self._acc_sums, seed=seed)
+            self.plan.backward(saved, gouts, False, self.grad_views, sums_arena=self._acc_sums, seed=seed,
+                               batch_reduce=gb)
             if self.world > 1:
                 self._allreduce(0, self.arena.numel())
             self._optim_range(0, self.arena.numel(), l1)
+        if gb is not None:
+            # the reported loss and correct count of the global batch (the other loss paths reduced theirs already)
+            if self.loss == "ce" and head >= 0:
+                self._reduce_f64(self._acc_ce[0:1])
+            self._reduce_i64(self._acc_corr)
         self.kernels_per_step = ops.launch_count() - k0
         return sums, l1, corr
 
@@ -372,12 +419,16 @@ class TrainStep:
             feat, wt = saved[0][nd.src], nd.conv.weight.detach()
             bias = None if nd.conv.bias is None else nd.conv.bias.detach()
             ops.head_dice_fwd(feat, wt, bias, y, self.dice_sums, self._acc_corr)
+            if self._batch_reduce is not None:
+                self._reduce_f64(self.dice_sums)
             dfeat = ops.head_dice_train(feat, wt, bias, y, w, self.dice_sums, eps, self._acc_ce,
                                         self.grad_views[id(nd.conv.weight)],
                                         None if nd.conv.bias is None else self.grad_views[id(nd.conv.bias)])
             return {nd.src: dfeat}, [None]
         logits = outs[0]
         ops.dice_fwd(logits, y, sums=self.dice_sums)
+        if self._batch_reduce is not None:
+            self._reduce_f64(self.dice_sums)
         ops.ce_fwd(logits, y, None, want_correct=True, sums=self._acc_spare, corr=self._acc_corr)
         ops.dice_loss(self.dice_sums, w, eps, self._acc_ce)
         return None, [ops.dice_bwd(logits, y, w, self.dice_sums, eps)]
@@ -390,6 +441,9 @@ class TrainStep:
         total = CE + l1_decay*l1_sum."""
         self.model.train()
         self.plan.epoch += 1  # parameters / BN buffers change under raw kernels (also on graph replay)
+        if self.global_batch and self.world > 1 and self._shard_shape != (tuple(x.shape), tuple(y.shape)):
+            check_equal_shards(x, y, self.pg)  # once per input shape: before a capture, or eagerly
+            self._shard_shape = (tuple(x.shape), tuple(y.shape))
         if not self.use_graph:
             x = x.to(self.dev, non_blocking=True)
             y = y.to(self.dev, non_blocking=True)
@@ -480,6 +534,34 @@ class TrainStep:
         if self.peer is not None:
             self.peer.check()
         return num / den + self.l1_decay * float(self.l1_sum)
+
+
+class _RankReduce:
+    """Plan.forward / Plan.backward's `batch_reduce` of a global-batch TrainStep: in-place sums and means over the
+    ranks of float64 slices of the step's accumulator buffer, on the current stream."""
+
+    def __init__(self, ts: TrainStep):
+        self.world = ts.world
+        self._ts = ts
+
+    def sum(self, buf: torch.Tensor) -> None:
+        self._ts._reduce_f64(buf)
+
+    def mean(self, buf: torch.Tensor) -> None:
+        self._ts._reduce_f64(buf, 1.0 / self.world)
+
+
+def check_equal_shards(x: torch.Tensor, y: torch.Tensor, group=None) -> None:
+    """A global batch divides by world * (this rank's count) and averages the BatchNorm backward sums, which is right
+    only if every rank holds as many samples of the same size: compare the input shapes of all ranks (one
+    all_gather_object; collective) and raise ValueError on every rank if they differ."""
+    dist = torch.distributed
+    mine = (tuple(x.shape), tuple(y.shape))
+    every = [None] * dist.get_world_size(group)
+    dist.all_gather_object(every, mine, group=group)
+    if any(e != every[0] for e in every):
+        raise ValueError(f"TrainStep(global_batch=True): every rank must hold the same shard shape, got "
+                         f"(x, y) shapes {every}")
 
 
 class _HostPipe:
